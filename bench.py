@@ -8,7 +8,7 @@ streams the weights from HBM) plus the RMSNorm / SiLU*mul glue kernels that keep
 Attention, KV cache, embeddings and lm_head are not on the path (BASELINE.json north_star:
 "awq/modules/fused/* sits unchanged on top", "synthetic Llama-shape activations").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--mode decode|prefill] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--mode decode|prefill] [--impl reference] [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0).  value = whole-job tokens/s with inputs resident in HBM (CUDA-graph
 replay of the plugin calls); e2e = the same step driven from pinned HOST buffers through the
@@ -25,6 +25,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -286,96 +287,20 @@ def cpu_reference_sample(M, layers_sample, reps, threads=None):
     return min(ts), cores
 
 
+def dump_outputs(directory, y, max_elems=4096 * 1024):
+    """The output of the last timed step, [M, 4096], as DIR/output.npy in float32.  The inputs and weights come from
+    seeded generators, so two builds run with the same arguments can be compared file for file.  A prefill output
+    (M = 4096) is larger than 64 MB in float32: then a fixed, seeded sample of rows is written, with their indices in
+    DIR/output_rows.npy."""
+    import numpy as np
 
-# ------------------------------------------------------------------- same-box GPU reference (Triton) leg
-def _load_reference_triton():
-    """The reference's own in-tree GPU kernels (awq/modules/triton/gemm.py: awq_gemm_triton :310-359,
-    awq_dequantize_triton :255-302), loaded BY FILE from the unmodified copy in baseline/_ref (installed by
-    __graft_entry__.build(); the file needs only torch + triton).  Measurement infrastructure: nothing of it is
-    on the product path."""
-    import importlib.util
-
-    for base in (os.path.join(ROOT, "baseline", "_ref"), "/root/reference"):
-        f = os.path.join(base, "awq", "modules", "triton", "gemm.py")
-        if os.path.isfile(f):
-            spec = importlib.util.spec_from_file_location("ref_triton_gemm", f)
-            mod = importlib.util.module_from_spec(spec)
-            spec.loader.exec_module(mod)
-            return mod
-    return None
-
-
-def triton_reference_leg(torch, rep, M, steps, warmup):
-    """What the unmodified reference runs on this box when `awq_ext` is absent (awq/modules/linear/gemm.py:60-69):
-    decode -> awq_gemm_triton(x, qweight, scales, qzeros, split_k_iters=8) per linear; prefill (B*S >= 1024) ->
-    awq_dequantize_triton + torch.matmul.  Same packed tensors as our arm, CUDA events, graph replay when the
-    launches capture.  Also the max error of both arms against the fp64 oracle contraction on one linear
-    (SURVEY 7.3: our error must not exceed the reference's)."""
-    T = _load_reference_triton()
-    if T is None:
-        return {"unavailable": "no copy of the reference on this box (baseline/_ref missing)"}
-    out = {"source": "awq/modules/triton/gemm.py (unmodified, baseline/_ref)",
-           "path": "awq_gemm_triton split_k=8" if M * 1 < 1024 else "awq_dequantize_triton + torch.matmul"}
-    xk = {HIDDEN: rep.xn, INTER: rep.act}
-
-    def lin(K, w):
-        x = xk[K]
-        if M >= 1024:   # gemm.py:61-65
-            return torch.matmul(x, T.awq_dequantize_triton(w[0], w[1], w[2]))
-        return T.awq_gemm_triton(x, w[0], w[1], w[2], 8)
-
-    def step():
-        for lw in rep.w:
-            for name, K, _N in LINEARS:
-                lin(K, lw[name])
-
-    try:
-        step()   # JIT
-        torch.cuda.synchronize()
-    except Exception as ex:  # noqa: BLE001
-        return {"unavailable": f"reference Triton path failed on this box: {type(ex).__name__}: {str(ex)[:160]}"}
-    fn, graphed = step, False
-    try:
-        g, _ = capture(torch, step)
-        fn, graphed = g.replay, True
-    except Exception:  # noqa: BLE001
-        torch.cuda.synchronize()
-    sec = timed(torch, fn, steps, warmup)
-    out.update({"tok_s": round(M * steps / sec, 2), "ms_per_step": round(sec / steps * 1e3, 4), "cuda_graph": graphed,
-                "launch_note": "linears only (128 per step), no glue kernels"})
-    per = {}
-    for name, K, _N in LINEARS:
-        def shape_step(name=name, K=K):
-            for lw in rep.w:
-                lin(K, lw[name])
-        try:
-            gs, _ = capture(torch, shape_step)
-            f2 = gs.replay
-        except Exception:  # noqa: BLE001
-            f2 = shape_step
-        t = timed(torch, f2, max(3, steps // 3), 2)
-        per[name] = round(t / max(3, steps // 3) / len(rep.w) * 1e6, 2)
-    out["per_linear_us"] = per
-    # error of both arms vs the fp64 oracle on layer 0's o-projection (4096 x 4096), at most 64 tokens
-    try:
-        import numpy as np
-
-        from oracle import awq_oracle as O
-
-        qw, sc, qz = rep.w[0]["o"]
-        w64 = O.dequantize_gemm(qw.cpu().numpy(), qz.cpu().numpy(), sc.cpu().numpy(), GROUP).astype(np.float64)
-        xm = rep.xn[: min(M, 64)].contiguous()
-        ref = xm.cpu().numpy().astype(np.float64) @ w64
-        rms = float(np.sqrt(np.mean(ref**2))) or 1.0
-        y_t = (torch.matmul(xm, T.awq_dequantize_triton(qw, sc, qz)) if M >= 1024
-               else T.awq_gemm_triton(xm, qw, sc, qz, 8)).float().cpu().numpy()
-        y_o = rep.lin(xm, (qw, sc, qz)).float().cpu().numpy()
-        out["max_err_over_rms"] = {"reference_triton": float(np.abs(y_t - ref).max() / rms),
-                                   "ours": float(np.abs(y_o - ref).max() / rms),
-                                   "on": f"o_proj 4096x4096 layer 0, {xm.shape[0]} token(s), fp64 oracle contraction"}
-    except Exception as ex:  # noqa: BLE001
-        out["max_err_over_rms"] = {"error": str(ex)[:160]}
-    return out
+    os.makedirs(directory, exist_ok=True)
+    y = y.float().cpu().numpy().reshape(-1, y.shape[-1])
+    rows = np.arange(y.shape[0])
+    if y.size > max_elems:
+        rows = np.sort(np.random.default_rng(0).choice(y.shape[0], max_elems // y.shape[1], replace=False))
+    np.save(os.path.join(directory, "output.npy"), np.ascontiguousarray(y[rows]))
+    np.save(os.path.join(directory, "output_rows.npy"), rows.astype(np.float64))
 
 
 def gemv_4096_leg(torch, ext, dev, steps, peaks):
@@ -758,8 +683,10 @@ def main():
     ap.add_argument("--layers", type=int, default=LAYERS, help="debug only: fewer layers => INVALID as a bench value")
     ap.add_argument("--tp-layers", type=int, default=0, help="debug: layers of the tensor-parallel leg (0 = all 80)")
     ap.add_argument("--legs", type=int, default=1,
-                    help="1: also run the secondary legs at N=1 (reference Triton on the same box, 4096x4096 GEMV, "
-                         "prefill); 0: headline only")
+                    help="1: also run the secondary legs at N=1 (4096x4096 GEMV, small batch, prefill, Mixtral); "
+                         "0: headline only")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the output of the last timed step to DIR/output.npy (float32) for comparing builds")
     a = ap.parse_args()
     a.warmup = max(a.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
@@ -819,7 +746,7 @@ def main():
             os.environ["NCCL_DEBUG"] = "INFO"
             os.environ.setdefault("NCCL_DEBUG_SUBSYS", "INIT,GRAPH")
         if "NCCL_DEBUG_FILE" not in os.environ:      # (a caller's own NCCL log file wins)
-            logdir = os.path.join(ROOT, "gpurun_out") if os.path.isdir(os.path.join(ROOT, "gpurun_out")) else "/tmp"
+            logdir = tempfile.gettempdir()
             os.environ["NCCL_DEBUG_FILE"] = os.path.join(logdir, "nccl_bench.%h.%p.log")
             nccl_log = os.path.join(logdir, f"nccl_bench.{os.uname().nodename}.{os.getpid()}.log")
         import torch.distributed as dist
@@ -880,6 +807,8 @@ def main():
     t_wall0 = time.time()
     sec = timed(torch, g_step.replay, a.steps, a.warmup, dist)
     t_wall1 = time.time()
+    if rank == 0 and a.dump_outputs:
+        dump_outputs(a.dump_outputs, out_static)
     clocks = None
     if rank == 0:
         t_ext = None
@@ -1016,10 +945,9 @@ def main():
     n_eager = max(3, a.steps // 5)
     sec_eager = timed(torch, eager_step, n_eager, 2, dist)
 
-    # secondary legs (N = 1 only; the headline metric is unchanged): the reference's Triton kernels on the same box,
-    # the metric's own 4096 x 4096 GEMV, and config 3 (prefill) - all CUDA-event timed like the value leg
+    # secondary legs (N = 1 only; the headline metric is unchanged): the metric's own 4096 x 4096 GEMV, small batches,
+    # config 3 (prefill) and Mixtral - all CUDA-event timed like the value leg
     if world == 1 and a.legs:
-        config["triton_reference"] = triton_reference_leg(torch, rep, M, max(5, a.steps // 2), 3)
         if a.mode == "decode":
             config["gemv_4096"] = gemv_4096_leg(torch, rep.ext, dev, a.steps, peaks)
             config["small_batch"] = small_batch_leg(torch, rep.ext, dev, a.steps, peaks)

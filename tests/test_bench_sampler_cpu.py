@@ -55,7 +55,7 @@ def test_nvml_sampler_extension_is_reported(monkeypatch):
     assert out["samples_in_timed_region"] < 3 <= out["samples"] and "note" in out and out["reasons"] == []
 
 
-def test_sampler_falls_back_when_nvml_is_unusable(monkeypatch):
+def test_sampler_falls_back_when_nvml_is_unusable(monkeypatch, tmp_path):
     broken = types.ModuleType("pynvml")
 
     def boom():
@@ -63,8 +63,9 @@ def test_sampler_falls_back_when_nvml_is_unusable(monkeypatch):
 
     broken.nvmlInit = boom
     monkeypatch.setitem(sys.modules, "pynvml", broken)
+    monkeypatch.setenv("PATH", str(tmp_path))      # and no nvidia-smi, even on a GPU machine
     bench = importlib.import_module("bench")
     s = bench.ClockSampler(0)
-    s.start()                                      # nvidia-smi is absent here too: both paths must degrade quietly
+    s.start()                                      # nvidia-smi is absent too: both paths must degrade quietly
     out = s.stop(time.time() - 1, time.time())
     assert out["sm_mhz"] is None and "samples" in out or out["reasons"]

@@ -1,14 +1,13 @@
-"""The drop-in, exercised for real: the UNMODIFIED reference package (tests/_refload.py: baseline/_ref, installed by
-`__graft_entry__.build()`) imported with this repo's `awq_ext` / `awq_v2_ext` on the path, so that the reference's
-own module classes - WQLinear_GEMM / GEMV / GEMVFast (awq/modules/linear/*.py), WQLinearMMFunction incl. backward
-(gemm.py:24-114), FasterTransformerRMSNorm (fused/norm.py:19-38), fuse_qkv (utils/fused_utils.py:45-142),
-apply_moe_weights (fused/moe.py:45-89) and the loader `from_quantized` / `_load_quantized_modules`
-(models/base.py:409-570,634-685) - run on the B200 kernels.  Results are compared with the CPU oracle (fp64
-contraction of the bit-exact dequantised weights), not with this repo's mirrors.
-
-Skipped (loudly) when no copy of the reference is reachable; on the GPU box `baseline/_ref` travels with the
-snapshot.
+"""The drop-in, exercised as the reference package (casper-hansen/AutoAWQ @ 88e4c76) calls it: tests/golden/
+dropin_calls.json holds every `awq_ext` / `awq_v2_ext` call that the reference's own module classes make - WQLinear_GEMM
+forward in every dispatch arm and backward (awq/modules/linear/gemm.py:24-298), WQLinear_GEMV / GEMVFast (gemv.py:27-197,
+gemv_fast.py:68-208), FasterTransformerRMSNorm (fused/norm.py:19-38), fuse_qkv (utils/fused_utils.py:45-142),
+apply_moe_weights, fused_topk and moe_align_block_size (fused/moe.py:45-170) - recorded by tests/golden/
+make_dropin_calls.py: function, argument order, scalars, tensor shapes / dtypes and where each tensor comes from.
+These tests rebuild the same seeded inputs, replay the calls on this repository's extension modules and compare the
+results with the CPU oracle (fp64 contraction of the bit-exact dequantised weights), not with this repo's mirrors.
 """
+import hashlib
 import json
 import os
 
@@ -18,12 +17,12 @@ import torch
 
 from oracle import awq_oracle as O
 
-import _refload
-
 pytestmark = pytest.mark.gpu
 
 RTOL, WR_GEMV, WR_TC = 2.0**-10, 2.0**-11, 2.0**-16
-ROOT = _refload.ROOT
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+_DT = {"float16": torch.float16, "bfloat16": torch.bfloat16, "float32": torch.float32, "int16": torch.int16,
+       "int32": torch.int32}
 
 
 def _dev():
@@ -32,6 +31,10 @@ def _dev():
 
 def _t(a):
     return torch.from_numpy(np.ascontiguousarray(a)).to(_dev())
+
+
+def _bits(a):
+    return np.ascontiguousarray(a).view(np.uint16)
 
 
 def _budget(x, w):
@@ -46,215 +49,228 @@ def _close(y, ref64, budget, wr, what=""):
 
 
 @pytest.fixture(scope="module")
-def ref():
-    awq = _refload.load_reference(shim=True)
-    if awq is None:
-        pytest.skip("no copy of the reference reachable (baseline/_ref missing: run __graft_entry__.build() in the "
-                    "build container before shipping)")
-    import awq.modules.linear.gemm as G
-    import awq.modules.linear.gemv as V
-    import awq.modules.linear.gemv_fast as F
-
-    # the reference bound THIS repo's extension modules (awq/utils/module.py:4-9)
-    for mod, name in ((G.awq_ext, "awq_ext"), (V.awq_ext, "awq_ext"), (F.awq_v2_ext, "awq_v2_ext")):
-        assert mod is not None and mod.__name__ == name
-        assert os.path.abspath(mod.__file__).startswith(ROOT + os.sep), mod.__file__
-    assert not os.path.abspath(awq.__file__).startswith(os.path.join(ROOT, "autoawq_b200"))
-    return awq
+def calls():
+    with open(os.path.join(GOLDEN, "dropin_calls.json")) as f:
+        return json.load(f)
 
 
-def _fill_gemm(m, c):
-    m.qweight.copy_(_t(c["qweight"]))
-    m.qzeros.copy_(_t(c["qzeros"]))
-    m.scales.copy_(_t(c["scales"]))
+def _segments(calls, scenario):
+    return {s["label"]: s for s in calls["segments"][scenario]}
+
+
+def _replay(segment, inputs):
+    """Makes the recorded calls of one segment on this repository's awq_ext / awq_v2_ext, with the tensors built from
+    `inputs` (name -> tensor), from earlier calls' results, or as the reference allocated them.  Returns one
+    (args, result) pair per call."""
+    import awq_ext
+    import awq_v2_ext
+
+    mods = {"awq_ext": awq_ext, "awq_v2_ext": awq_v2_ext}
+    done = []
+    for c in segment["calls"]:
+        args = []
+        for a in c["args"]:
+            if "v" in a:
+                args.append(a["v"])
+                continue
+            shape, dt = tuple(a["shape"]), _DT[a["dtype"]]
+            if "in" in a:
+                t = inputs[a["in"]].to(dt).reshape(shape)
+            elif "call" in a:
+                prev_args, prev_ret = done[a["call"]]
+                t = prev_ret if a["arg"] == "ret" else prev_args[a["arg"]]
+                assert tuple(t.shape) == shape and t.dtype == dt, (c["fn"], a)
+            elif "values" in a:
+                t = torch.tensor(a["values"], dtype=dt, device=_dev()).reshape(shape)
+            elif "fill" in a:
+                t = torch.full(shape, a["fill"], dtype=dt, device=_dev())
+            else:
+                t = torch.empty(shape, dtype=dt, device=_dev())
+            args.append(t)
+        ret = getattr(mods[c["mod"]], c["fn"])(*args)
+        if c["ret"] is None:
+            assert ret is None, c["fn"]
+        else:
+            assert tuple(ret.shape) == tuple(c["ret"]["shape"]) and ret.dtype == _DT[c["ret"]["dtype"]], c["fn"]
+        done.append((args, ret))
+    torch.cuda.synchronize()
+    return done
+
+
+def _gemm_inputs(c):
+    return {"qweight": _t(c["qweight"]), "scales": _t(c["scales"]), "qzeros": _t(c["qzeros"])}
 
 
 # ------------------------------------------------------------------ WQLinear_GEMM (gemm.py:116-298), all dispatch arms
 @pytest.mark.parametrize("K,N,G", [(512, 256, 128), (1024, 1792, 128), (4096, 4096, 128), (256, 64, 64)])
-def test_reference_wqlinear_gemm_forward(ref, K, N, G):
-    from awq.modules.linear.gemm import WQLinear_GEMM
-
+def test_reference_wqlinear_gemm_forward(calls, K, N, G):
+    segs = _segments(calls, f"gemm_forward_{K}_{N}_{G}")
     c = O.make_case(K, N, G, seed=K + N)
     w = O.dequantize_gemm(c["qweight"], c["qzeros"], c["scales"], G)
+    inputs = _gemm_inputs(c)
     rng = np.random.default_rng(3)
-    bias = (rng.standard_normal(N) * 0.25).astype(np.float16)
-    m = WQLinear_GEMM(4, G, K, N, True, _dev())
-    _fill_gemm(m, c)
-    m.bias.copy_(_t(bias))
     # [1,1,K] / [1,8,K]: gemm_forward_cuda (gemm.py:56-58); [1,40,K]: same entry, tensor-core kernel;
     # [2,600,K]: B*S >= 1024 -> dequantize_weights_cuda + torch.matmul (gemm.py:50-54); 2-D: M*K >= 1024 -> same
-    for shape in [(1, 1, K), (1, 8, K), (1, 40, K), (2, 600, K), (3, K)]:
-        x = (rng.standard_normal(shape) * 0.5).astype(np.float16)
-        y = m(_t(x))
-        assert y.dtype == torch.float16 and tuple(y.shape) == shape[:-1] + (N,)
+    cases = [((1, 1, K), np.float16), ((1, 8, K), np.float16), ((1, 40, K), np.float16), ((2, 600, K), np.float16),
+             ((3, K), np.float16), ((2, 3, K), None)]
+    for shape, dt in cases:
+        label = str(shape) if dt is not None else "bf16 (2, 3, K)"
+        if dt is None:   # a bf16 input: the module casts it to fp16 before the call (gemm.py:43)
+            xt = torch.randn(shape, device=_dev(), dtype=torch.bfloat16)
+            x = xt.half().cpu().numpy()
+        else:
+            x = (rng.standard_normal(shape) * 0.5).astype(np.float16)
+            xt = _t(x)
+        [(args, y)] = _replay(segs[label], dict(inputs, x=xt))
         x2 = x.reshape(-1, K)
-        nb = O.gemm_f64(x2, w)
-        ref64 = (nb + bias.astype(np.float64)).reshape(shape[:-1] + (N,))
-        Mtot = x2.shape[0]
-        # the dequant+cuBLAS arm rounds like the tensor-core path; allow cuBLAS fp16 accumulation slack there
-        wr = WR_GEMV if Mtot <= 8 else (2.0**-11 if len(shape) == 2 or shape[0] * shape[1] >= 1024 else WR_TC)
-        # the reference module adds the bias AFTER the kernel, in fp16 (gemm.py:79): a second rounding, of size
-        # 2^-11 |x.W| on the kernel's own output, on top of the final one - both inside this budget
-        bud = _budget(x2, w) * wr + 2.0**-10 * (np.abs(nb) + np.abs(bias.astype(np.float64)))
-        _close(y.cpu().numpy(), ref64, bud.reshape(ref64.shape), 1.0, f"ref WQLinear_GEMM {shape}")
-    # dtype round trip + empty batch (gemm.py:44-45,256-258,284-285)
-    xb = torch.randn(2, 3, K, device=_dev(), dtype=torch.bfloat16)
-    assert m(xb).dtype == torch.bfloat16
-    assert tuple(m(torch.zeros(0, 2, K, device=_dev(), dtype=torch.float16)).shape) == (0, 2, N)
+        if segs[label]["calls"][0]["fn"] == "dequantize_weights_cuda":
+            # the reference multiplies by the dequantised weight itself: the extension's part is that weight, bit for bit
+            assert np.array_equal(_bits(y.cpu().numpy()), _bits(w)), f"dequantize_weights_cuda {shape}"
+        else:
+            wr = WR_GEMV if x2.shape[0] <= 8 else WR_TC
+            _close(y.cpu().numpy().reshape(x2.shape[0], N), O.gemm_f64(x2, w), _budget(x2, w), wr,
+                   f"ref WQLinear_GEMM {shape}")
+    # an empty batch returns before any extension call (gemm.py:44-45)
+    assert segs["empty batch"]["calls"] == []
 
 
-def test_reference_from_linear_then_forward(ref):
-    """The reference packer (gemm.py:171-251) on the GPU, then its forward on our kernels."""
-    from awq.modules.linear.gemm import WQLinear_GEMM
-
+def test_reference_from_linear_then_forward(calls):
+    """The reference packer (gemm.py:171-251) gave exactly the oracle's packed buffers; its forward on our kernels."""
     K, N, G = 256, 128, 64
     rng = np.random.default_rng(0)
     iw, iz, s = O.quantize_rtn((rng.standard_normal((N, K)) * 0.05).astype(np.float32), G)
-    wq = O.dequantize_gemm(*O.pack_gemm(iw, iz), s, G)
-    lin = torch.nn.Linear(K, N, bias=False).half()
-    lin.weight.data = torch.from_numpy(wq.T.copy())
-    m = WQLinear_GEMM.from_linear(lin.to(_dev()), 4, G, False, _t(s.astype(np.float16)), _t(iz.astype(np.float16)))
-    assert np.array_equal(m.qweight.cpu().numpy(), O.pack_gemm(iw, iz)[0])
+    qw, qz = O.pack_gemm(iw, iz)
+    packed = {"qweight": qw, "scales": s.astype(np.float16), "qzeros": qz}
+    for name, a in packed.items():
+        assert hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest() == calls["from_linear_sha256"][name], name
+    wq = O.dequantize_gemm(qw, qz, s, G)
     x = (rng.standard_normal((1, 5, K))).astype(np.float16)
-    _close(m.to(_dev())(_t(x)).cpu().numpy()[0], O.gemm_f64(x[0], wq), _budget(x[0], wq), WR_GEMV, "from_linear fwd")
+    [(_, y)] = _replay(calls["segments"]["from_linear"][0], dict({k: _t(v) for k, v in packed.items()}, x=_t(x)))
+    _close(y.cpu().numpy().reshape(5, N), O.gemm_f64(x[0], wq), _budget(x[0], wq), WR_GEMV, "from_linear fwd")
 
 
-def test_reference_backward(ref):
+def test_reference_backward(calls):
     """WQLinearMMFunction.backward (gemm.py:88-114): dX = dY . W^T through awq_ext.dequantize_weights_cuda(…,1,0,0,False);
-    no weight gradient.  Driven through the reference module in training mode, and through this repo's mirror."""
-    from awq.modules.linear.gemm import WQLinear_GEMM
+    no weight gradient.  Replayed as the reference module calls it in training mode, and through this repo's mirror."""
     from autoawq_b200.linear import WQLinear_GEMM as Mirror
 
     K, N, G = 512, 256, 128
     c = O.make_case(K, N, G, seed=9)
-    w = O.dequantize_gemm(c["qweight"], c["qzeros"], c["scales"], G).astype(np.float64)
+    w16 = O.dequantize_gemm(c["qweight"], c["qzeros"], c["scales"], G)
+    w = w16.astype(np.float64)
     rng = np.random.default_rng(4)
     x = (rng.standard_normal((2, 6, K)) * 0.5).astype(np.float16)
     gy = (rng.standard_normal((2, 6, N)) * 0.5).astype(np.float16)
     ref_gx = gy.astype(np.float64) @ w.T
-    for cls in (WQLinear_GEMM, Mirror):
-        m = cls(4, G, K, N, False, _dev(), training=True) if cls is WQLinear_GEMM else cls(4, G, K, N, False, _dev())
-        m.training = True
-        _fill_gemm(m, c)
-        xt = _t(x).requires_grad_(True)
-        y = m(xt)
-        assert y.requires_grad
-        y.backward(_t(gy))
-        gx = xt.grad.float().cpu().numpy()
-        assert gx.shape == x.shape
-        tol = 2.0**-9 * np.abs(ref_gx) + 2.0**-10 * (np.abs(gy.astype(np.float64)) @ np.abs(w.T)) + 1e-4
-        assert np.all(np.abs(gx - ref_gx) <= tol), f"{cls.__module__}: max err {np.abs(gx - ref_gx).max():.3e}"
+    (_, y), (_, wd) = _replay(calls["segments"]["backward"][0], dict(_gemm_inputs(c), x=_t(x)))
+    x2 = x.reshape(-1, K)
+    _close(y.cpu().numpy(), O.gemm_f64(x2, w16), _budget(x2, w16), WR_TC, "training forward")
+    assert np.array_equal(_bits(wd.cpu().numpy()), _bits(w16)), "backward's dequantised weight"
+    m = Mirror(4, G, K, N, False, _dev())
+    m.training = True
+    m.qweight.copy_(_t(c["qweight"]))
+    m.qzeros.copy_(_t(c["qzeros"]))
+    m.scales.copy_(_t(c["scales"]))
+    xt = _t(x).requires_grad_(True)
+    y = m(xt)
+    assert y.requires_grad
+    y.backward(_t(gy))
+    gx = xt.grad.float().cpu().numpy()
+    assert gx.shape == x.shape
+    tol = 2.0**-9 * np.abs(ref_gx) + 2.0**-10 * (np.abs(gy.astype(np.float64)) @ np.abs(w.T)) + 1e-4
+    assert np.all(np.abs(gx - ref_gx) <= tol), f"mirror: max err {np.abs(gx - ref_gx).max():.3e}"
 
 
 # ----------------------------------------------------------- WQLinear_GEMV / GEMVFast (gemv.py:27-197, gemv_fast.py:68-208)
 @pytest.mark.parametrize("K,N,G", [(512, 128, 128), (4096, 512, 128), (1024, 256, 64)])
-def test_reference_wqlinear_gemv_and_fast_forward(ref, K, N, G):
-    from awq.modules.linear.gemv import WQLinear_GEMV
-    from awq.modules.linear.gemv_fast import WQLinear_GEMVFast
-
+def test_reference_wqlinear_gemv_and_fast_forward(calls, K, N, G):
+    segs = _segments(calls, f"gemv_{K}_{N}_{G}")
     c = O.make_case(K, N, G, seed=K)
     w = O.dequantize_gemm(c["qweight"], c["qzeros"], c["scales"], G)
     vw, vz, vs = O.pack_gemv(c["intweight"], c["zeros"], c["scales"], G)
     fw, fs, fz = O.pack_gemv_fast(c["intweight"], c["zeros"], c["scales"], G)
     wfast = O.dequantize_gemv_fast_f64(fw, fs, fz, G)
-    mv = WQLinear_GEMV(4, G, K, N, False, _dev())
-    mv.qweight.copy_(_t(vw)); mv.qzeros.copy_(_t(vz)); mv.scales.copy_(_t(vs))
-    mf = WQLinear_GEMVFast(4, G, K, N, False, _dev())
-    mf.qweight.copy_(_t(fw)); mf.qzeros.copy_(_t(fz)); mf.scales.copy_(_t(fs))
     rng = np.random.default_rng(1)
     # GEMV module: M <= 8 -> gemv_forward_cuda, M > 8 -> gemmv2_forward_cuda (gemv.py:168-180)
     for shape in [(1, 1, K), (2, 4, K), (1, 24, K)]:
         x = (rng.standard_normal(shape) * 0.5).astype(np.float16)
         x2 = x.reshape(-1, K)
-        y = mv(_t(x)).cpu().numpy()
-        assert y.shape == shape[:-1] + (N,)
-        _close(y.reshape(-1, N), O.gemm_f64(x2, w), _budget(x2, w), WR_GEMV if x2.shape[0] <= 8 else WR_TC,
-               f"ref WQLinear_GEMV {shape}")
+        [(_, y)] = _replay(segs[f"gemv {shape}"], {"qweight": _t(vw), "qzeros": _t(vz), "scales": _t(vs), "x": _t(x)})
+        _close(y.cpu().numpy().reshape(-1, N), O.gemm_f64(x2, w), _budget(x2, w),
+               WR_GEMV if x2.shape[0] <= 8 else WR_TC, f"ref WQLinear_GEMV {shape}")
     # GEMVFast module: batch < 8 and one token -> decode kernel, else prefill (gemv_fast.py:185-208)
     for shape in [(1, 1, K), (4, 1, K), (1, 20, K), (9, 1, K)]:
         x = (rng.standard_normal(shape) * 0.5).astype(np.float16)
         x2 = x.reshape(-1, K)
-        y = mf(_t(x)).cpu().numpy()
-        assert y.shape == shape[:-1] + (N,)
-        _close(y.reshape(-1, N), O.gemm_f64(x2, wfast), _budget(x2, wfast), WR_GEMV, f"ref WQLinear_GEMVFast {shape}")
+        [(_, y)] = _replay(segs[f"fast {shape}"], {"qweight": _t(fw), "qzeros": _t(fz), "scales": _t(fs), "x": _t(x)})
+        assert tuple(y.shape) == shape[:-1] + (N,)
+        _close(y.cpu().numpy().reshape(-1, N), O.gemm_f64(x2, wfast), _budget(x2, wfast), WR_GEMV,
+               f"ref WQLinear_GEMVFast {shape}")
 
 
 # ----------------------------------------------------------------------------- fused modules that call awq_ext bare
-def test_reference_fastertransformer_rmsnorm(ref):
-    from awq.modules.fused.norm import FasterTransformerRMSNorm
-
+def test_reference_fastertransformer_rmsnorm(calls):
+    segs = _segments(calls, "rmsnorm")
     rng = np.random.default_rng(2)
     for shape in [(1, 1, 4096), (2, 7, 512)]:
         x = rng.standard_normal(shape).astype(np.float16)
         wgt = (1 + 0.1 * rng.standard_normal(shape[-1])).astype(np.float16)
-        out = FasterTransformerRMSNorm(_t(wgt), eps=1e-5)(_t(x))
-        np.testing.assert_allclose(out.cpu().numpy(), O.rmsnorm_f64(x.reshape(-1, shape[-1]), wgt, 1e-5).reshape(shape),
-                                   rtol=2e-3, atol=2e-3)
+        [(args, _)] = _replay(segs[str(shape)], {"x": _t(x), "weight": _t(wgt)})
+        np.testing.assert_allclose(args[2].cpu().numpy(),
+                                   O.rmsnorm_f64(x.reshape(-1, shape[-1]), wgt, 1e-5).reshape(shape), rtol=2e-3, atol=2e-3)
 
 
 @pytest.mark.parametrize("version", ["gemm", "gemv", "gemv_fast"])
-def test_reference_fuse_qkv(ref, version):
-    """fuse_qkv (fused_utils.py:45-142) concatenates the packed buffers; the fused module on our kernels must give
-    [q | k | v] of the separate projections' oracle outputs."""
-    from awq.modules.linear.gemm import WQLinear_GEMM
-    from awq.modules.linear.gemv import WQLinear_GEMV
-    from awq.modules.linear.gemv_fast import WQLinear_GEMVFast
-    from awq.utils.fused_utils import fuse_qkv
-
+def test_reference_fuse_qkv(calls, version):
+    """fuse_qkv (fused_utils.py:45-142) concatenates the packed buffers (along the axes it used, as recorded); the fused
+    module on our kernels must give [q | k | v] of the separate projections' oracle outputs."""
     K, G = 512, 128
     widths = (512, 128, 128)
-    projs, ws = [], []
+    parts, ws = {"qweight": [], "scales": [], "qzeros": []}, []
     for i, N in enumerate(widths):
         c = O.make_case(K, N, G, seed=40 + i)
         if version == "gemm":
-            m = WQLinear_GEMM(4, G, K, N, False, _dev())
-            _fill_gemm(m, c)
+            bufs = (c["qweight"], c["scales"], c["qzeros"])
             ws.append(O.dequantize_gemm(c["qweight"], c["qzeros"], c["scales"], G))
         elif version == "gemv":
             vw, vz, vs = O.pack_gemv(c["intweight"], c["zeros"], c["scales"], G)
-            m = WQLinear_GEMV(4, G, K, N, False, _dev())
-            m.qweight.copy_(_t(vw)); m.qzeros.copy_(_t(vz)); m.scales.copy_(_t(vs))
+            bufs = (vw, vs, vz)
             ws.append(O.dequantize_gemm(c["qweight"], c["qzeros"], c["scales"], G))
         else:
             fw, fs, fz = O.pack_gemv_fast(c["intweight"], c["zeros"], c["scales"], G)
-            m = WQLinear_GEMVFast(4, G, K, N, False, _dev())
-            m.qweight.copy_(_t(fw)); m.qzeros.copy_(_t(fz)); m.scales.copy_(_t(fs))
+            bufs = (fw, fs, fz)
             ws.append(O.dequantize_gemv_fast_f64(fw, fs, fz, G))
-        projs.append(m)
-    holder = torch.nn.Module()
-    holder.q_proj, holder.k_proj, holder.v_proj = projs
-    qkv = fuse_qkv(holder, *projs)
-    assert qkv.out_features == sum(widths)
+        for name, b in zip(("qweight", "scales", "qzeros"), bufs):
+            parts[name].append(b)
+    axes = calls["fuse_qkv_axes"][version]
+    inputs = {name: _t(np.concatenate(ps, axis=axes[name])) for name, ps in parts.items()}
     w = np.concatenate(ws, axis=1)
     x = (np.random.default_rng(5).standard_normal((1, 1, K)) * 0.5).astype(np.float16)
-    y = qkv(_t(x)).cpu().numpy().reshape(1, -1)
-    _close(y, O.gemm_f64(x.reshape(1, K), w), _budget(x.reshape(1, K), w), WR_GEMV, f"fuse_qkv {version}")
+    [(_, y)] = _replay(calls["segments"][f"fuse_qkv_{version}"][0], dict(inputs, x=_t(x)))
+    assert y.shape[-1] == sum(widths)
+    _close(y.cpu().numpy().reshape(1, -1), O.gemm_f64(x.reshape(1, K), w), _budget(x.reshape(1, K), w), WR_GEMV,
+           f"fuse_qkv {version}")
 
 
-def test_reference_apply_moe_weights(ref):
+def test_reference_apply_moe_weights(calls):
     """apply_moe_weights (fused/moe.py:45-89): fused_topk -> moe_align_block_size -> grouped_gemm_forward ->
     silu_and_mul -> grouped_gemm_forward(mul_weights) -> sum, all through our awq_ext."""
-    from awq.modules.fused.moe import apply_moe_weights
-    from awq.utils.fused_utils import fuse_linears  # noqa: F401  (imports cleanly with the shim)
-
     E, K, I, G, T, topk = 4, 512, 1024, 128, 3, 2
-
-    class W:
-        pass
-
     rng = np.random.default_rng(6)
-    w1, w2, W1, W2 = W(), W(), [], []
-    c1 = [O.make_case(K, 2 * I, G, seed=60 + e) for e in range(E)]
-    c2 = [O.make_case(I, K, G, seed=70 + e) for e in range(E)]
-    for dst, cs, store in ((w1, c1, W1), (w2, c2, W2)):
-        dst.qweight = _t(np.stack([c["qweight"] for c in cs]))
-        dst.qzeros = _t(np.stack([c["qzeros"] for c in cs]))
-        dst.scales = _t(np.stack([c["scales"] for c in cs]))
+    inputs, W1, W2 = {}, [], []
+    for tag, cs, store in (("w1", [O.make_case(K, 2 * I, G, seed=60 + e) for e in range(E)], W1),
+                           ("w2", [O.make_case(I, K, G, seed=70 + e) for e in range(E)], W2)):
+        for b in ("qweight", "qzeros", "scales"):
+            inputs[f"{tag}.{b}"] = _t(np.stack([c[b] for c in cs]))
         for c in cs:
             store.append(O.dequantize_gemm(c["qweight"], c["qzeros"], c["scales"], G).astype(np.float64))
     x = (rng.standard_normal((T, K)) * 0.5).astype(np.float16)
     logits = rng.standard_normal((T, E)).astype(np.float32)
-    y = apply_moe_weights(w1, w2, _t(x), _t(logits), topk, renormalize=True).float().cpu().numpy()
+    done = _replay(calls["segments"]["moe"][0], dict(inputs, x=_t(x), logits=_t(logits)))
+    # our topk_softmax, renormalised as fused_topk does (moe.py:169-170), gives the weights the reference passed on
+    tw = done[0][0][0]
+    assert torch.allclose(tw / tw.sum(dim=-1, keepdim=True), done[2][0][4], rtol=1e-5, atol=1e-6)
+    y = torch.sum(done[-1][1], dim=1).float().cpu().numpy()      # the reference's final reduction (moe.py:89)
     p = np.exp(logits - logits.max(-1, keepdims=True))
     p /= p.sum(-1, keepdims=True)
     ref_y = np.zeros((T, K))
@@ -269,150 +285,37 @@ def test_reference_apply_moe_weights(ref):
     assert np.all(np.abs(y - ref_y) <= tol), np.abs(y - ref_y).max()
 
 
-# ----------------------------------------------------------- the loader: from_quantized / _load_quantized_modules
-def _tiny_checkpoint(tmp_path, version="gemm"):
-    """A 2-layer Llama-shaped AWQ checkpoint directory (config.json + model.safetensors), random-init packed
-    weights; returns (path, dict name -> dense fp16 weight [K, N] for the twin)."""
-    from safetensors.torch import save_file
-
-    H, I, L, V, heads, kv, G = 256, 512, 2, 320, 4, 2, 64
-    cfg = {
-        "architectures": ["LlamaForCausalLM"], "model_type": "llama", "hidden_size": H, "intermediate_size": I,
-        "num_hidden_layers": L, "num_attention_heads": heads, "num_key_value_heads": kv, "head_dim": H // heads,
-        "vocab_size": V, "rms_norm_eps": 1e-5, "max_position_embeddings": 128, "rope_theta": 10000.0,
-        "hidden_act": "silu", "tie_word_embeddings": False, "torch_dtype": "float16", "attention_bias": False,
-        "mlp_bias": False,
-        "quantization_config": {"quant_method": "awq", "zero_point": True, "group_size": G, "bits": 4,
-                                "version": version, "modules_to_not_convert": None},
-    }
-    os.makedirs(tmp_path, exist_ok=True)
-    with open(os.path.join(tmp_path, "config.json"), "w") as f:
-        json.dump(cfg, f)
-    rng = np.random.default_rng(11)
-    sd, dense = {}, {}
-    dk = H // heads
-    shapes = {"self_attn.q_proj": (H, H), "self_attn.k_proj": (H, kv * dk), "self_attn.v_proj": (H, kv * dk),
-              "self_attn.o_proj": (H, H), "mlp.gate_proj": (H, I), "mlp.up_proj": (H, I), "mlp.down_proj": (I, H)}
-    for l in range(L):
-        for name, (K, N) in shapes.items():
-            c = O.make_case(K, N, G, seed=100 * l + len(name))
-            sc = (c["scales"].astype(np.float32) / (6.1 * 0.0108 * np.sqrt(K))).astype(np.float16)
-            p = f"model.layers.{l}.{name}"
-            sd[p + ".qweight"] = torch.from_numpy(c["qweight"])
-            sd[p + ".qzeros"] = torch.from_numpy(c["qzeros"])
-            sd[p + ".scales"] = torch.from_numpy(sc)
-            dense[p] = O.dequantize_gemm(c["qweight"], c["qzeros"], sc, G)
-        for nm in ("input_layernorm", "post_attention_layernorm"):
-            sd[f"model.layers.{l}.{nm}.weight"] = torch.from_numpy((1 + 0.05 * rng.standard_normal(H)).astype(np.float16))
-    sd["model.embed_tokens.weight"] = torch.from_numpy((rng.standard_normal((V, H)) * 0.5).astype(np.float16))
-    sd["model.norm.weight"] = torch.from_numpy((1 + 0.05 * rng.standard_normal(H)).astype(np.float16))
-    sd["lm_head.weight"] = torch.from_numpy((rng.standard_normal((V, H)) * 0.05).astype(np.float16))
-    save_file(sd, os.path.join(tmp_path, "model.safetensors"))
-    return str(tmp_path), cfg, sd, dense
-
-
-def _dispatch(model, checkpoint, device_map=None, **kw):
-    """Stands in for accelerate.load_checkpoint_and_dispatch (base.py:527-535): materialise the meta model on
-    cuda:0 and fill every parameter / buffer from the safetensors file."""
-    from safetensors.torch import load_file
-
-    sd = load_file(os.path.join(checkpoint, "model.safetensors"))
-    model.to_empty(device="cuda:0")
-    missing = []
-    own = dict(model.named_parameters())
-    own.update(dict(model.named_buffers()))
-    with torch.no_grad():
-        for k, v in own.items():
-            if k in sd:
-                v.copy_(sd[k].to(v.dtype))
-            elif "rotary" in k or "inv_freq" in k:
-                pass
-            else:
-                missing.append(k)
-    assert not missing, missing
-    # rotary inv_freq buffers were created on meta: recompute them
-    for mod in model.modules():
-        if hasattr(mod, "inv_freq") and hasattr(mod, "config"):
-            fn = getattr(mod, "rope_init_fn", None) or getattr(mod, "compute_default_rope_parameters")
-            inv, _ = fn(mod.config, torch.device("cuda:0"))
-            mod.inv_freq = inv
-            if hasattr(mod, "original_inv_freq"):
-                mod.original_inv_freq = inv.clone()
-    return model
-
-
-def test_reference_from_quantized_unfused(ref, tmp_path):
-    """AutoAWQForCausalLM.from_quantized -> BaseAWQForCausalLM._load_quantized_modules replaces every nn.Linear of
-    the decoder layers with the reference's WQLinear_GEMM (base.py:634-685), which then runs on our awq_ext.
-    Logits vs a dense fp16 twin built from the oracle-dequantised weights."""
-    _refload.stub_accelerate(dispatch=_dispatch)
-    import awq.models.base as B
-    from awq import AutoAWQForCausalLM
-    from awq.modules.linear.gemm import WQLinear_GEMM
-    from transformers import LlamaConfig, LlamaForCausalLM
-
-    B.load_checkpoint_and_dispatch = _dispatch  # the stub installed at import time, re-pointed at the real filler
-    path, cfg, sd, dense = _tiny_checkpoint(tmp_path / "ckpt")
-    model = AutoAWQForCausalLM.from_quantized(path, fuse_layers=False, safetensors=True, device_map="balanced")
-    n_q = sum(isinstance(m, WQLinear_GEMM) for m in model.model.modules())
-    assert n_q == 7 * cfg["num_hidden_layers"]
-    twin_cfg = LlamaConfig(**{k: v for k, v in cfg.items() if k not in ("quantization_config", "architectures")})
-    twin = LlamaForCausalLM(twin_cfg).half().to(_dev())
-    tsd = {}
-    for k, v in sd.items():
-        if k.endswith(".qweight"):
-            p = k[: -len(".qweight")]
-            tsd[p + ".weight"] = torch.from_numpy(dense[p].T.copy())
-        elif not k.endswith((".qzeros", ".scales")):
-            tsd[k] = v
-    missing, unexpected = twin.load_state_dict(tsd, strict=False)
-    assert not [m for m in missing if "rotary" not in m and "inv_freq" not in m], missing
-    ids = torch.tensor([[1, 5, 17, 42, 99, 7]], device=_dev())
-    with torch.no_grad():
-        a = model.model(ids).logits.float()
-        b = twin(ids).logits.float()
-    assert a.shape == b.shape
-    err = (a - b).abs().max().item()
-    assert err <= 3e-2 * b.abs().max().item() + 2e-2, f"logits differ: {err} (max |ref| {b.abs().max().item()})"
-    # a single-token step (the decode shape): every linear is one awq_ext.gemm_forward_cuda call
-    with torch.no_grad():
-        a1 = model.model(ids[:, :1]).logits.float()
-        b1 = twin(ids[:, :1]).logits.float()
-    assert (a1 - b1).abs().max().item() <= 3e-2 * b1.abs().max().item() + 2e-2
-
-
-def test_reference_fused_topk_both_branches_agree(ref, monkeypatch):
+def test_reference_fused_topk_both_branches_agree(calls):
     """The reference itself holds a second definition of `topk_softmax`: on ROCm `fused_topk` computes
-    `torch.softmax` + `torch.topk` instead of calling the extension (awq/modules/fused/moe.py:150-153).  Running the
-    reference's own function through both branches - the extension branch lands in OUR awq_ext.topk_softmax - pins
-    the operator to reference code rather than to this repository's reading of it.  Same for the renormalisation."""
-    import awq.modules.fused.moe as M
-
+    `torch.softmax` + `torch.topk` instead of calling the extension (awq/modules/fused/moe.py:150-153).  That branch's
+    routing, recorded from the reference's own function, must equal the extension branch run on OUR
+    awq_ext.topk_softmax - which pins the operator to reference code rather than to this repository's reading of it.
+    Same for the renormalisation."""
+    segs = calls["segments"]["fused_topk"]
     rng = np.random.default_rng(12)
-    for (T, E, topk) in [(1, 8, 2), (7, 8, 2), (33, 64, 6), (5, 60, 4)]:
-        logits = torch.from_numpy(rng.standard_normal((T, E)).astype(np.float32)).to(_dev())
-        w_ext, id_ext = M.fused_topk(logits, topk, renormalize=True)
-        monkeypatch.setattr(torch.version, "hip", "reference-rocm-branch", raising=False)
-        try:
-            w_ref, id_ref = M.fused_topk(logits, topk, renormalize=True)
-        finally:
-            monkeypatch.setattr(torch.version, "hip", None, raising=False)
-        assert torch.equal(id_ext.long(), id_ref.long()), (T, E, topk)
+    for seg, want, (T, E, topk) in zip(segs, calls["fused_topk_torch_branch"], [(1, 8, 2), (7, 8, 2), (33, 64, 6),
+                                                                              (5, 60, 4)]):
+        logits = rng.standard_normal((T, E)).astype(np.float32)
+        [(args, _)] = _replay(seg, {"logits": _t(logits)})
+        w_ext = args[0] / args[0].sum(dim=-1, keepdim=True)          # renormalize=True (moe.py:169-170)
+        w_ref = torch.tensor(want["weights"], dtype=torch.float32, device=_dev())
+        id_ref = torch.tensor(want["ids"], dtype=torch.int64, device=_dev())
+        assert torch.equal(args[1].long(), id_ref), (T, E, topk)
         assert torch.allclose(w_ext, w_ref, rtol=1e-5, atol=1e-7)
 
 
-def test_reference_moe_align_block_size_invariants(ref):
+def test_reference_moe_align_block_size_invariants(calls):
     """moe_align_block_size through the reference's wrapper (moe.py:92-134), at sizes beyond its docstring example:
     every expert's run is a multiple of the block, holds exactly that expert's slots in ascending order, padding slots
     carry `numel`, expert_ids name the run's expert."""
-    import awq.modules.fused.moe as M
-
+    segs = calls["segments"]["moe_align"]
     rng = np.random.default_rng(13)
-    for (T, E, topk, block) in [(4, 4, 3, 4), (1, 8, 2, 16), (37, 8, 2, 16), (100, 60, 4, 16)]:
+    for seg, (T, E, topk, block) in zip(segs, [(4, 4, 3, 4), (1, 8, 2, 16), (37, 8, 2, 16), (100, 60, 4, 16)]):
         ids = np.stack([rng.permutation(E)[:topk] for _ in range(T)]).astype(np.int32)
-        s_ids, e_ids, npost = M.moe_align_block_size(torch.from_numpy(ids).to(_dev()), block, E)
-        n = int(npost.item())
-        s_ids, e_ids = s_ids.cpu().numpy()[:n], e_ids.cpu().numpy()[: n // block]
+        [(args, _)] = _replay(seg, {"ids": _t(ids)})
+        assert args[1:3] == [E, block]
+        n = int(args[5].item())
+        s_ids, e_ids = args[3].cpu().numpy()[:n], args[4].cpu().numpy()[: n // block]
         assert n % block == 0
         flat = ids.reshape(-1)
         pos = 0
