@@ -23,6 +23,8 @@ struct NvtxScope {
 
 static std::atomic<int> g_knobs[32] = {{0}, {0}, {8}};   // (the rest value-initialise to 0)
 int knob(int key) { return (key >= 0 && key < 32) ? g_knobs[key].load(std::memory_order_relaxed) : 0; }
+// keys b200awq_set_knob accepts (include/b200awq.h lists them); any other key is an error rather than a silent no-op
+static constexpr uint32_t kLiveKnobs = 0x7fu /* 0-6 */ | 1u << 12 | 1u << 14 | 1u << 15 | 1u << 16 | 1u << 19 | 1u << 21;
 
 NvtxScope::NvtxScope(const char* name) : on(knob(15) != 0) {
   if (on) nvtxRangePushA(name);
@@ -89,7 +91,7 @@ size_t b200awq_workspace_bytes(int M, int K, int N) {
 }
 
 int b200awq_set_knob(int key, int value) {
-  if (key < 0 || key >= 32) return B200AWQ_EINVAL;
+  if (key < 0 || key >= 32 || ((kLiveKnobs >> key) & 1u) == 0) return B200AWQ_EINVAL;
   g_knobs[key].store(value, std::memory_order_relaxed);
   if (key == 16) return fold(program_set_watchdog_seconds(value));   // decode-program watchdog (device-side constant)
   return B200AWQ_OK;

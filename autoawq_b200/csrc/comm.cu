@@ -6,20 +6,21 @@
 // (profiles/r02_tp70b_n2.json) - 3.6 ms of a 9.9 ms step.  This kernel does the same sum in one launch of one CTA:
 //
 //   every rank owns a SYMMETRIC buffer (cudaMalloc + CUDA IPC: each process maps all peers' buffers):
-//       inbox[2 parities][world slots][max_elems] fp16, flags[2][world] u32
+//       inbox[2 parities][world slots][max_elems / 2] LL words of 8 bytes = {two fp16 values, 32-bit call number}
 //   call number e (a device-resident counter: CUDA-graph replay safe), parity p = e & 1, rank r:
-//     1. push: store my partial into slot r of EVERY rank's inbox[p] (P2P stores over NVLink / NVSwitch, 16-byte
-//        vectors; the own copy is a local store),
-//     2. signal: after a CTA barrier, thread q does fence.sys + st.release.sys flags[p][r] = e on rank q,
-//     3. wait: thread q spins (ld.acquire.sys) until my flags[p][q] == e - all partials have landed here,
-//     4. reduce: every thread sums its vector over the slots in RANK ORDER (fp32 accumulation, one rounding): the
-//        result is bit-identical on all ranks, and written over the partial in place.
+//     1. push: store my partial, as LL words tagged e, into slot r of EVERY rank's inbox[p] (P2P stores over NVLink /
+//        NVSwitch; the own copy is a local store),
+//     2. wait and reduce: every thread polls its words of each slot of my inbox[p] until they carry e, and sums them in
+//        RANK ORDER (fp32 accumulation, one rounding): the result is bit-identical on all ranks, and written over the
+//        partial in place.
+//   Every word carries its own validity (NCCL's LL idea): ONE NVLink hop, no barrier, no fence, no flag.  8-byte
+//   aligned stores do not tear; 16-byte vectors (two words) are used on both sides.  (A flag protocol - push, CTA
+//   barrier, fence.sys, flag store, flag poll, reduce - measured 8.1 us at N = 2 against 5.2 us for LL,
+//   profiles/r02_tp70b_n2.json.)
 //   Two parities: a rank can start call e + 1 (writing inbox[(e + 1) & 1]) while a slower peer still reads
-//   inbox[e & 1]; it cannot start e + 2 before every peer has signalled e + 1, i.e. finished reading e.
+//   inbox[e & 1]; it cannot start e + 2 before every peer has pushed e + 1, i.e. finished reading e.
 //   No memset, no host round trip, nothing to reset.  A spin gives up after 2 s (dead peer) and raises the comm's
 //   error flag instead of hanging the GPU.
-// The DEFAULT protocol is the LL variant further down (data words that carry their own validity: one hop, no fence);
-// the flag protocol described here is kept behind knob 17 for comparison.
 //
 // Messages larger than the buffer (prefill) stay on NCCL (autoawq_b200/comm.py decides).
 #include <cuda_fp16.h>
@@ -50,95 +51,10 @@ struct Comm {
   size_t bytes = 0;
 };
 
-__host__ __device__ inline size_t comm_inbox_bytes(int world, int max_elems) {
-  return (size_t)2 * world * max_elems * sizeof(__half);
-}
-__host__ __device__ inline size_t comm_bytes(int world, int max_elems) {
-  // flag protocol: inbox + flags[2][<= 32] u32; LL protocol: 2 x the inbox (every 4 data bytes travel with 4 epoch bytes)
-  return 2 * comm_inbox_bytes(world, max_elems) + 2 * 128;
+static size_t comm_bytes(int world, int max_elems) {
+  return (size_t)2 * world * max_elems * 4;   // inbox[2][world][max_elems / 2] words of 8 bytes
 }
 
-__device__ __forceinline__ void st_release_sys_u32(uint32_t* p, uint32_t v) {
-  asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-}
-__device__ __forceinline__ uint32_t ld_acquire_sys_u32(const uint32_t* p) {
-  uint32_t v;
-  asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-
-__global__ void __launch_bounds__(kCommThreads, 1)
-    oneshot_allreduce_kernel(CommPeers peers, int rank, int world, int max_elems, __half* __restrict__ y, int n,
-                             int* __restrict__ state) {
-  const int tid = threadIdx.x;
-  const uint32_t e = (uint32_t)state[0] + 1u;
-  const int par = (int)(e & 1u);
-  const int nv = n >> 3;                                    // 16-byte vectors
-  const size_t slot_bytes = (size_t)max_elems * sizeof(__half);
-  const size_t inbox_off = (size_t)par * world * slot_bytes;
-  const size_t flags_off = comm_inbox_bytes(world, max_elems) + (size_t)par * 128;
-  // 1. push my partial into slot `rank` of every rank's inbox
-  const uint4* src = reinterpret_cast<const uint4*>(y);
-  for (int v = tid; v < nv; v += kCommThreads) {
-    const uint4 val = src[v];
-    for (int p = 0; p < world; ++p)
-      reinterpret_cast<uint4*>(peers.base[p] + inbox_off + (size_t)rank * slot_bytes)[v] = val;
-  }
-  __syncthreads();
-  // 2. signal every rank (release at system scope: cumulative over what the barrier ordered before it)
-  if (tid < world) {
-    __threadfence_system();
-    st_release_sys_u32(reinterpret_cast<uint32_t*>(peers.base[tid] + flags_off) + rank, e);
-  }
-  // 3. wait until every rank's partial has landed here
-  if (tid < world) {
-    const uint32_t* f = reinterpret_cast<const uint32_t*>(peers.base[rank] + flags_off) + tid;
-    unsigned long long t0 = 0;
-    int spins = 0;
-    while (ld_acquire_sys_u32(f) != e) {
-      if ((++spins & 1023) == 0) {
-        unsigned long long now;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now));
-        if (t0 == 0) t0 = now;
-        else if (now - t0 > 2000000000ull) {   // 2 s: a peer is gone - do not hang the GPU
-          state[1] = 1;
-          break;
-        }
-      }
-    }
-  }
-  __syncthreads();
-  // 4. reduce in rank order (same order everywhere: identical results on all ranks)
-  const uint8_t* mine = peers.base[rank] + inbox_off;
-  uint4* dst = reinterpret_cast<uint4*>(y);
-  for (int v = tid; v < nv; v += kCommThreads) {
-    float acc[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-    for (int q = 0; q < world; ++q) {
-      const uint4 val = reinterpret_cast<const uint4*>(mine + (size_t)q * slot_bytes)[v];
-      const __half2* h = reinterpret_cast<const __half2*>(&val);
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        const float2 f = __half22float2(h[j]);
-        acc[2 * j] += f.x;
-        acc[2 * j + 1] += f.y;
-      }
-    }
-    uint4 o;
-    __half2* oh = reinterpret_cast<__half2*>(&o);
-#pragma unroll
-    for (int j = 0; j < 4; ++j) oh[j] = __floats2half2_rn(acc[2 * j], acc[2 * j + 1]);
-    dst[v] = o;
-  }
-  if (tid == 0) state[0] = (int)e;
-}
-
-// ---------------------------------------------------------------------------------------------- LL protocol
-// The flag protocol above pays for: push, CTA barrier, fence.sys, flag store, flag poll, CTA barrier, reduce - two
-// NVLink hops and two fences in sequence (8.1 us at N = 2, 11.6 us at N = 8).  Here every 8-byte word carries its own
-// validity (NCCL's LL idea): {two fp16 values, 32-bit call number}.  A rank stores such words straight into every
-// peer's slot and polls its own slots word by word until the call number matches: ONE hop, no barrier, no fence, no
-// flag.  8-byte aligned stores do not tear; 16-byte vectors (two words) are used on both sides.  Same parity
-// double-buffering and device-resident call counter as above; same rank-ordered fp32 sum.
 __device__ __forceinline__ void st_relaxed_sys_u4(void* p, const uint4& v) {
   asm volatile("st.relaxed.sys.global.v4.u32 [%0], {%1, %2, %3, %4};" ::"l"(p), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
 }
@@ -250,14 +166,8 @@ cudaError_t comm_open(Comm* c, const void* handles) {
 }
 
 cudaError_t comm_all_reduce(Comm* c, void* y, int n, cudaStream_t st) {
-  // knob 17 = 1: the flag protocol (kept for comparison); default: LL words (one hop, no fences).  The two protocols
-  // share the buffer and the call counter but not their data layout: do not switch between calls that are in flight.
-  if (knob(17) == 1)
-    oneshot_allreduce_kernel<<<1, kCommThreads, 0, st>>>(c->peers, c->rank, c->world, c->max_elems, static_cast<__half*>(y),
-                                                         n, c->d_state);
-  else
-    ll_allreduce_kernel<<<1, kCommThreads, 0, st>>>(c->peers, c->rank, c->world, c->max_elems, static_cast<__half*>(y), n,
-                                                    c->d_state);
+  ll_allreduce_kernel<<<1, kCommThreads, 0, st>>>(c->peers, c->rank, c->world, c->max_elems, static_cast<__half*>(y), n,
+                                                  c->d_state);
   return cudaGetLastError();
 }
 

@@ -230,10 +230,6 @@ __device__ __forceinline__ void tma_prefetch_l2_2d(const void* tmap, int c0, int
 __device__ __forceinline__ void prefetch_l2_line(const void* gsrc) {
   asm volatile("prefetch.global.L2 [%0];" ::"l"(gsrc) : "memory");
 }
-// L2 prefetch of a contiguous range (size % 16 == 0), no completion tracking
-__device__ __forceinline__ void bulk_prefetch_l2(const void* gsrc, uint32_t bytes) {
-  asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(gsrc), "r"(bytes) : "memory");
-}
 // 1-D bulk copy global -> smem (no tensor map), completion on mbarrier (bytes); size % 16 == 0
 __device__ __forceinline__ void bulk_load_1d(void* smem_dst, const void* gsrc, uint32_t bytes, uint64_t* bar) {
   asm volatile(

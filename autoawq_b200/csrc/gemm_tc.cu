@@ -537,7 +537,7 @@ __global__ void __launch_bounds__(tc_threads<LAYOUT>(), 1)
 //     whole K column stores fp16 directly, a partial one adds fp32 into the caller's zeroed workspace and bumps the
 //     tile's ticket by its number of k-step pairs; the contributor that completes K rounds, adds the bias, restores
 //     zeros.  Wherever N / 128 <= SM count (and from 64 tokens on) the ranges are tile-aligned instead: gemm_tcq_grid.
-//   * knob 22 = optional HBM -> L2 prefetch ahead of the ring: measured, no gain (profiles/r02_tcq_knob20.json).
+//   * no HBM -> L2 prefetch ahead of the ring: measured, no gain (profiles/r02_tcq_knob20.json).
 template <int BT>
 struct TcqCfg {
   static constexpr int kNS = 4;                                            // A stages (producers -> MMA), 2 per team
@@ -613,7 +613,7 @@ __global__ void __launch_bounds__(TcqCfg<BT>::kThreads, 1)
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   pdl_trigger();
-  const bool dbg = (p.dbg & 1) != 0 && blockIdx.x < 256;
+  const bool dbg = p.dbg != 0 && blockIdx.x < 256;
   unsigned long long* dbg_row = g_tcq_dbg + blockIdx.x * 8;
   if (dbg && threadIdx.x == 0) dbg_row[0] = tcq_timer();
 
@@ -664,7 +664,6 @@ __global__ void __launch_bounds__(TcqCfg<BT>::kThreads, 1)
       const bool leader = elect_one();
       const uint32_t NW = (uint32_t)p.N >> 3;
       const uint32_t tx = (uint32_t)Cfg::kQTileBytes + (uint32_t)ng * 320u;
-      const int pf_ahead = p.ksplit;   // (field reused by this kernel: L2 prefetch distance in pairs)
       int qs = 0;
       uint32_t qph = 0;
       for (int t = t_begin; t < t_end;) {
@@ -675,14 +674,6 @@ __global__ void __launch_bounds__(TcqCfg<BT>::kThreads, 1)
           uint8_t* dst = q_base + (size_t)qs * Cfg::kQStageBytes;
           const uint32_t g = (uint32_t)(d * Cfg::kQRows) >> p.g_shift;
           if (leader) {
-            // optional HBM -> L2 prefetch of the pair pf_ahead positions further down this CTA's range (knob 22)
-            if (pf_ahead > 0) {
-              const int tp = t + (d - d0) + pf_ahead;
-              if (tp < t_end) {
-                const int ntp = tp / KP;
-                tma_prefetch_l2_2d(&tmq, ntp * 16, (tp - ntp * KP) * Cfg::kQRows);
-              }
-            }
             mbar_arrive_expect_tx(&qfull[qs], tx);
             tma_load_2d(dst, &tmq, &qfull[qs], nt * 16, d * Cfg::kQRows);
             for (int h = 0; h < ng; ++h) {
@@ -733,7 +724,6 @@ __global__ void __launch_bounds__(TcqCfg<BT>::kThreads, 1)
       constexpr uint32_t idesc = umma_idesc_f16(kTileN, BT, 1, 0);
       const int mw = warp == 1 ? 0 : 1;
       const bool leader = elect_one();
-      const int mma_per_step = (p.dbg & 8) ? 0 : ((p.dbg & 16) ? 1 : kBK / 16);
       const uint32_t a_base_s = smem_u32(a_base), x_base_s = smem_u32(x_base);
       const uint64_t da0 = umma_smem_desc(a_base_s, 8192, 1024);   // MN-major SW128; start address in bits [0, 14)
       const uint64_t db0 = umma_smem_desc(x_base_s, 16, 1024);     // K-major SW128
@@ -758,9 +748,8 @@ __global__ void __launch_bounds__(TcqCfg<BT>::kThreads, 1)
           if (leader) {
 #pragma unroll
             for (int k16 = 0; k16 < kBK / 16; ++k16)
-              if (k16 < mma_per_step)   // (4 unless a timing experiment is on: knob 20)
-                umma_f16_ss(d_tmem, da + (uint64_t)(k16 * (2048 >> 4)), db + (uint64_t)(k16 * (32 >> 4)), idesc,
-                            (d > d0 || k16 > 0) ? 1u : 0u);
+              umma_f16_ss(d_tmem, da + (uint64_t)(k16 * (2048 >> 4)), db + (uint64_t)(k16 * (32 >> 4)), idesc,
+                          (d > d0 || k16 > 0) ? 1u : 0u);
             umma_commit(&empty[stage]);
             umma_commit(&xempty[xs]);
           }
@@ -890,8 +879,8 @@ __global__ void __launch_bounds__(TcqCfg<BT>::kThreads, 1)
         fetch(nxt, qs_n);
       }
       mbar_wait(&empty[stage], phase ^ 1);
-      if (!(p.dbg & 2)) cur.store(p, 0, 0, dt, a_base_s + (uint32_t)stage * kAStageBytes);   // (timing experiment: knob 20)
-      if (!(p.dbg & 4)) fence_proxy_async_smem();   // every writer: generic-proxy stores -> visible to the tensor core
+      cur.store(p, 0, 0, dt, a_base_s + (uint32_t)stage * kAStageBytes);
+      fence_proxy_async_smem();   // every writer: generic-proxy stores -> visible to the tensor core
       __syncwarp();
       if (lane == 0) {
         mbar_arrive(&full[stage]);
@@ -1120,9 +1109,8 @@ cudaError_t gemm_tc(const GemmArgs& a, int layout, float* acc_ws, int* tickets, 
     const int BQ = a.M <= 16 ? 16 : (a.M <= 32 ? 32 : (a.M <= 64 ? 64 : 128));
     CUtensorMap tmxq, tmwq;
     p.m_tiles = 1;
-    p.ksplit = knob(22);   // small-M kernel: L2 prefetch distance in k-step pairs (0 = off)
     p.has_tmq = 1;
-    p.dbg = (knob(3) == 9 ? 1 : 0) | ((knob(20) & 15) << 1);   // knob 20: timing experiments (results invalid)
+    p.dbg = knob(3) == 9 ? 1 : 0;
     cudaError_t eq = make_x_tmap(a.x, a.ldx, a.M, a.K, BQ, &tmxq);
     if (eq == cudaSuccess)
       eq = make_tmap_2d(a.qweight, 1, (uint64_t)(a.N / 8), (uint64_t)a.K, (uint64_t)(a.N / 8) * 4, 16, 2 * kBK, &tmwq, false);

@@ -334,13 +334,13 @@ struct V3Moe {
   int n_slots, topk, x_per_slot, block_size;
 };
 
-template <int MT, int SPW, bool XS, bool MOE = false>
+template <int MT, int SPW, bool MOE = false>
 __global__ void __launch_bounds__(kV3Threads, 1)
     gemv_v3_kernel(const __grid_constant__ CUtensorMap tmw, const __half* __restrict__ x, int64_t ldx,
                    const __half* __restrict__ scales, const int32_t* __restrict__ qzeros,
                    const __half* __restrict__ bias, __half* __restrict__ y, float* __restrict__ acc_ws,
                    int* __restrict__ tickets, int M, int K, int N, int G, int g_shift,
-                   const uint8_t* __restrict__ next_w, long long next_bytes, int dbg, int l2_ahead, const V3Moe moe,
+                   const uint8_t* __restrict__ next_w, long long next_bytes, int dbg, const V3Moe moe,
                    int packed) {
   constexpr int NS = V3Smem<MT, SPW>::kStages;
   __shared__ int s_slot[8];       // MOE: output row of each of the job's slots (-1 = padding)
@@ -375,9 +375,6 @@ __global__ void __launch_bounds__(kV3Threads, 1)
   int* flags = reinterpret_cast<int*>(empty + NS);   // [0..7] per-warp push flags, [8] CTA flag,
   int* warp_cb = flags + 16;                         // [8] column block of each warp's pending sums
   int* warp_ntl = warp_cb + 8;                       // [8] tiles those sums cover
-  // XS: the activations of all MT tokens staged once per CTA (row stride K + 8 halves)
-  __half* xs = reinterpret_cast<__half*>(v3_smem + V3Smem<MT, SPW>::bytes);
-  const int xs_stride = K + 8;
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int NW = N >> 3;
@@ -413,23 +410,13 @@ __global__ void __launch_bounds__(kV3Threads, 1)
       const int w = lane;
       const int a = t0 + (int)((int64_t)ntile * w / kV3Warps);
       const int bnd = t0 + (int)((int64_t)ntile * (w + 1) / kV3Warps);
-      // Optional HBM -> L2 prefetch kL2Ahead tiles ahead of the shared-memory ring (knob 8).  Measured r1 (ring
-      // sweep in profiles/): no gain - 19.5 us without vs 20.7 us with it on 4096x28672 - the 24-stage ring already
-      // saturates what the consumers can drain, extra requests only lengthen the queues.  Default: off.
-      const int kL2Ahead = l2_ahead > 0 ? SPW + l2_ahead : 0;  // 0: no L2 prefetch
-      int cbp = a / TPC, ktp = a - cbp * TPC;      // prefetch cursor (no per-tile divisions)
-      auto pf_one = [&]() {
-        tma_prefetch_l2_2d(&tmw, cbp * (kV3TileCols / 8), row_off + ktp * kV3TileRows);
-        if (++ktp == TPC) { ktp = 0; ++cbp; }
-      };
-      for (int tp = a; tp < bnd && tp < a + kL2Ahead; ++tp) pf_one();
-      const bool do_pf = kL2Ahead > 0;
+      // No HBM -> L2 prefetch ahead of the ring: the 24-stage ring already saturates what the consumers can drain
+      // (19.5 us without vs 20.7 us with one on 4096 x 28672, profiles/r01_gemv_v3_ring_sweep.json).
       int cb = a / TPC, kt = a - cb * TPC;
       int stage_i = 0;
       uint32_t ph = 0;
       for (int t = a; t < bnd; ++t) {
         const int stage = w * SPW + stage_i;
-        if (do_pf && t + kL2Ahead < bnd) pf_one();
         mbar_wait(&empty[stage], ph ^ 1);
         const int grp_abs = (kt * kV3TileRows) >> g_shift;
         uint8_t* st = ring + (size_t)stage * kV3TileBytes;
@@ -486,35 +473,14 @@ __global__ void __launch_bounds__(kV3Threads, 1)
 #pragma unroll
     for (int bb = 0; bb < 4; ++bb) xb[bb][0] = xb[bb][1] = 0u;
     if (t < b_w && tok_ok) {
-      if (XS) {
-        const __half* px = xs + g * xs_stride + ktile * kV3TileRows + 2 * tig;
+      const __half* px = xrow + ktile * kV3TileRows + 2 * tig;
 #pragma unroll
-        for (int bb = 0; bb < 4; ++bb) {
-          xb[bb][0] = *reinterpret_cast<const uint32_t*>(px + 16 * bb);
-          xb[bb][1] = *reinterpret_cast<const uint32_t*>(px + 16 * bb + 8);
-        }
-      } else {
-        const __half* px = xrow + ktile * kV3TileRows + 2 * tig;
-#pragma unroll
-        for (int bb = 0; bb < 4; ++bb) {
-          xb[bb][0] = *reinterpret_cast<const uint32_t*>(px + 16 * bb);
-          xb[bb][1] = *reinterpret_cast<const uint32_t*>(px + 16 * bb + 8);
-        }
+      for (int bb = 0; bb < 4; ++bb) {
+        xb[bb][0] = *reinterpret_cast<const uint32_t*>(px + 16 * bb);
+        xb[bb][1] = *reinterpret_cast<const uint32_t*>(px + 16 * bb + 8);
       }
     }
   };
-  if (XS) {
-    // stage x[m][0..K) for the real tokens (16-byte chunks; K % 64 == 0, rows 8-byte aligned at least)
-    const int chunks = K / 8;
-    for (int i = ct; i < M * chunks; i += kV3Warps * 32) {
-      const int m = i / chunks, c8 = (i - m * chunks) * 8;
-      const __half* src = x + (int64_t)m * ldx + c8;
-      uint2 lo = *reinterpret_cast<const uint2*>(src), hi = *reinterpret_cast<const uint2*>(src + 4);
-      *reinterpret_cast<uint2*>(xs + m * xs_stride + c8) = lo;
-      *reinterpret_cast<uint2*>(xs + m * xs_stride + c8 + 4) = hi;
-    }
-    named_bar_sync_gv(1, kV3Warps * 32);
-  }
 
   float acc[4][4][4];
   float xs_acc[4];
@@ -685,7 +651,7 @@ static cudaError_t ensure_smem_attr(Kern kern, size_t smem, std::atomic<uint64_t
   return e;
 }
 
-template <int MT, int SPW, bool XS>
+template <int MT, int SPW>
 static cudaError_t launch_v3(const GemmArgs& a, float* acc_ws, int* tickets, cudaStream_t st) {
   const NextW nx = learn_successor(a.qweight, (long long)a.K * (a.N / 8) * 4);
   int g_shift = 31;  // G == K: a single group
@@ -698,23 +664,21 @@ static cudaError_t launch_v3(const GemmArgs& a, float* acc_ws, int* tickets, cud
   cudaError_t e = make_tmap_2d(a.qweight, /*int32*/ 1, (uint64_t)(a.N / 8), (uint64_t)a.K, (uint64_t)(a.N / 8) * 4, 32,
                                kV3TileRows, &tm);
   if (e != cudaSuccess) return e;
-  auto kern = gemv_v3_kernel<MT, SPW, XS>;
-  const size_t smem = V3Smem<MT, SPW>::bytes + (XS ? (size_t)MT * (a.K + 8) * 2 : 0);
+  auto kern = gemv_v3_kernel<MT, SPW>;
+  const size_t smem = V3Smem<MT, SPW>::bytes;
   static std::atomic<uint64_t> attr_done{0};
-  // (XS variants size their request by K: set the maximum once, launch with the exact size)
-  e = ensure_smem_attr(kern, XS ? (size_t)227 * 1024 : smem, attr_done);
+  e = ensure_smem_attr(kern, smem, attr_done);
   if (e != cudaSuccess) return e;
   const int T = (a.N / kV3TileCols) * (a.K / kV3TileRows);
   const int grid = T < v3_sm_count() ? T : v3_sm_count();
   return launch_kernel(kern, dim3(grid), dim3(kV3Threads), smem, st, tm, reinterpret_cast<const __half*>(a.x), a.ldx,
                        reinterpret_cast<const __half*>(a.scales), a.qzeros, reinterpret_cast<const __half*>(a.bias),
                        reinterpret_cast<__half*>(a.y), acc_ws, tickets, a.M, a.K, a.N, a.G, g_shift,
-                       reinterpret_cast<const uint8_t*>(nx.ptr), nx.bytes, knob(3) == 1 ? 1 : 0, knob(8) > 0 ? knob(8) - 1 : 0,
+                       reinterpret_cast<const uint8_t*>(nx.ptr), nx.bytes, knob(3) == 1 ? 1 : 0,
                        // packed epilogue at M = 1 only: there it saves the ticket and read-back round trips (4096 x 4096:
                        // 8.75 -> 7.18 us); for M >= 2 the returning 64-bit atomics cost more than they save on the
                        // larger shapes (4096 x 14336, M = 8: 32 -> 49 us), so those keep fp32 REDs + tickets.
-                       // knob 18 = 1: ticket epilogue everywhere
-                       V3Moe{}, (MT == 1 && a.K / kV3TileRows < 256 && knob(18) == 0) ? 1 : 0);
+                       V3Moe{}, (MT == 1 && a.K / kV3TileRows < 256) ? 1 : 0);
 }
 
 // Grouped launch: grid.y = sorted_len / 8 jobs (most of them padding: they exit at once).  Needs hbs * 8 rows of fp32
@@ -744,12 +708,12 @@ cudaError_t gemv_v3_moe(const void* x, int x_per_slot, const int32_t* qweight, c
     return launch_kernel(kern, dim3(grid, hbs), dim3(kV3Threads), smem, st, tm, reinterpret_cast<const __half*>(x),
                          (int64_t)K, reinterpret_cast<const __half*>(scales), qzeros, static_cast<const __half*>(nullptr),
                          reinterpret_cast<__half*>(y), acc_ws, tickets, mt, K, N, G, g_shift,
-                         static_cast<const uint8_t*>(nullptr), 0LL, 0, 0, moe, 0);   // (grouped jobs keep the ticket epilogue)
+                         static_cast<const uint8_t*>(nullptr), 0LL, 0, moe, 0);   // (grouped jobs keep the ticket epilogue)
   };
-  if (tokens <= 1) return go(gemv_v3_kernel<1, 3, false, true>, V3Smem<1, 3>::bytes, 1);
-  if (tokens <= 2) return go(gemv_v3_kernel<2, 2, false, true>, V3Smem<2, 2>::bytes, 2);
-  if (tokens <= 4) return go(gemv_v3_kernel<4, 2, false, true>, V3Smem<4, 2>::bytes, 4);
-  return go(gemv_v3_kernel<8, 2, false, true>, V3Smem<8, 2>::bytes, 8);
+  if (tokens <= 1) return go(gemv_v3_kernel<1, 3, true>, V3Smem<1, 3>::bytes, 1);
+  if (tokens <= 2) return go(gemv_v3_kernel<2, 2, true>, V3Smem<2, 2>::bytes, 2);
+  if (tokens <= 4) return go(gemv_v3_kernel<4, 2, true>, V3Smem<4, 2>::bytes, 4);
+  return go(gemv_v3_kernel<8, 2, true>, V3Smem<8, 2>::bytes, 8);
 }
 
 bool gemv_v3_moe_supported(int K, int N, int G, int hbs) {
@@ -766,21 +730,12 @@ bool gemv_v3_supported(const GemmArgs& a) {
 }
 
 cudaError_t gemv_v3(const GemmArgs& a, float* acc_ws, int* tickets, cudaStream_t st) {
-  constexpr size_t kMaxSmem = 227 * 1024;
-  if (a.M <= 1) {
-    // knob 7 = 1: stage the activations in shared memory (2 ring stages per warp instead of 3).  Measured r1:
-    // 477 vs 498 tok/s - the x loads were not the stall, the third stage is worth more.
-    if (knob(7) != 0 && V3Smem<1, 2>::bytes + (size_t)(a.K + 8) * 2 <= kMaxSmem) return launch_v3<1, 2, true>(a, acc_ws, tickets, st);
-    if (knob(9) == 1) return launch_v3<1, 1, false>(a, acc_ws, tickets, st);
-    if (knob(9) == 2) return launch_v3<1, 2, false>(a, acc_ws, tickets, st);
-    return launch_v3<1, 3, false>(a, acc_ws, tickets, st);
-  }
-  if (a.M <= 2) {
-    if (knob(7) != 0 && V3Smem<2, 2>::bytes + (size_t)2 * (a.K + 8) * 2 <= kMaxSmem) return launch_v3<2, 2, true>(a, acc_ws, tickets, st);
-    return launch_v3<2, 2, false>(a, acc_ws, tickets, st);
-  }
-  if (a.M <= 4) return launch_v3<4, 2, false>(a, acc_ws, tickets, st);
-  return launch_v3<8, 2, false>(a, acc_ws, tickets, st);   // (column sums in registers: two ring stages also at MT = 8)
+  // M = 1: three ring stages per warp (profiles/r01_gemv_v3_ring_sweep.json); activations come straight from global
+  // memory - staging them in shared memory cost the third stage and measured 477 vs 498 tok/s
+  if (a.M <= 1) return launch_v3<1, 3>(a, acc_ws, tickets, st);
+  if (a.M <= 2) return launch_v3<2, 2>(a, acc_ws, tickets, st);
+  if (a.M <= 4) return launch_v3<4, 2>(a, acc_ws, tickets, st);
+  return launch_v3<8, 2>(a, acc_ws, tickets, st);   // (column sums in registers: two ring stages also at MT = 8)
 }
 
 }  // namespace b200awq

@@ -57,8 +57,6 @@ struct __align__(128) ProgOp {
   int prologue;
   float eps;
   int ext_dep;            // >= 0: the external source was written by that (older) op of this program
-  int n_part;             // CTAs that share this op's tiles (the first n_part; 0 = all): small ops use fewer, so that
-                          // fewer CTAs add into each column block (knob 13 = minimum tiles per participating CTA)
   const int32_t* qw_src;  // the checkpoint-format qweight (host-side use: the stream variant re-lays it out)
 };
 static_assert(sizeof(ProgOp) == 256, "ProgOp layout");
@@ -69,7 +67,7 @@ __host__ __device__ constexpr size_t prog_fixed_smem(int spw) {
          (size_t)(kV3Warps * kProgMT * kGvRedStride + kV3Warps * kProgMT * kV3TileCols) * 4 +
          2 * kV3Warps * spw * 8 + 128 + 64;
 }
-static_assert(prog_fixed_smem(1) % 16 == 0 && prog_fixed_smem(2) % 16 == 0, "xs must stay 16-byte aligned");
+static_assert(prog_fixed_smem(2) % 16 == 0, "xs must stay 16-byte aligned");
 
 // knob 3 = 2: per-op phase timestamps (globaltimer ns) of the first 8 CTAs for the first 32 kernel ops:
 // [0] op begin, [1] previous op complete (wait over), [2] activations staged, [3] first tile landed (warp 0),
@@ -163,7 +161,7 @@ cudaError_t program_abort_clear(cudaStream_t st) {
   cudaError_t e = cudaGetSymbolAddress(&p, g_prog_abort);
   return e != cudaSuccess ? e : cudaMemsetAsync(p, 0, sizeof(g_prog_abort), st);
 }
-// watchdog limit in ns (default 0.5 s; knob 7 = seconds, for runs under compute-sanitizer / cuda-gdb where a kernel
+// watchdog limit in ns (default 0.5 s; knob 16 = seconds, for runs under compute-sanitizer / cuda-gdb where a kernel
 // is orders of magnitude slower and a healthy wait would be mistaken for a lost completion)
 __device__ unsigned long long g_prog_watch_ns = 500000000ull;
 cudaError_t program_set_watchdog_seconds(int seconds) {
@@ -245,7 +243,7 @@ constexpr int kProgThreads = kV3Threads + 32;   // producer warp + 8 consumer wa
 template <int SPW>
 __global__ void __launch_bounds__(kProgThreads, 1)
     program_kernel(const ProgOp* __restrict__ ops, int n_ops, unsigned long long* __restrict__ rows, int acc_stride,
-                   int* __restrict__ staged, int* __restrict__ zeroed, int M, int dbg, int gate, int backoff) {
+                   int* __restrict__ staged, int* __restrict__ zeroed, int M, int dbg) {
   constexpr int MT = kProgMT, NS = kV3Warps * SPW;
   extern __shared__ __align__(1024) uint8_t pg_smem[];
   uint8_t* ring = pg_smem;
@@ -302,17 +300,16 @@ __global__ void __launch_bounds__(kProgThreads, 1)
         const int NW = N >> 3;
         const int TPC = K / kV3TileRows;
         const int T = (N / kV3TileCols) * TPC;
-        const int np = o->n_part > 0 ? o->n_part : nblk;
-        const int t0 = bid < np ? (int)((int64_t)T * bid / np) : 0;
-        const int t1 = bid < np ? (int)((int64_t)T * (bid + 1) / np) : 0;
+        const int t0 = (int)((int64_t)T * bid / nblk);
+        const int t1 = (int)((int64_t)T * (bid + 1) / nblk);
         const int ntile = t1 - t0;
         const int a = t0 + (int)((int64_t)ntile * w / kV3Warps);
         const int bnd = t0 + (int)((int64_t)ntile * (w + 1) / kV3Warps);
         int cb = a / TPC, kt = a - cb * TPC;
-        // gate (knob 10): hold the next op's loads back until this CTA's sums of the previous op are on their way
+        // gate: hold the next op's loads back until this CTA's sums of the previous op are on their way
         // (measured +9 %: the REDs do not queue behind a fresh burst of bulk loads; the ring refills while the
         // consumers poll and stage)
-        if (gate && op > 0) prog_wait_smem(pub_op, op, kWGate, op);
+        if (op > 0) prog_wait_smem(pub_op, op, kWGate, op);
         for (int t = a; t < bnd; ++t) {
           const int stage = w * SPW + stage_i;
           if (!prog_mbar_wait(&empty[stage], ph ^ 1, kWEmpty, op)) return;
@@ -359,7 +356,7 @@ __global__ void __launch_bounds__(kProgThreads, 1)
         ProgWatch wd;
         while (!prog_prev8(R_prev, po->bias, c, TPCp, v)) {
           if (wd.tick(kWDutyY, i)) break;
-          if (backoff) __nanosleep(400);   // off the critical path: do not hammer the lines the REDs are landing on
+          __nanosleep(400);   // off the critical path: do not hammer the lines the REDs are landing on
         }
         *reinterpret_cast<uint4*>(po->y + c) = v;
       }
@@ -379,11 +376,11 @@ __global__ void __launch_bounds__(kProgThreads, 1)
               ProgWatch wd;
               while (!prog_prev8(pr, pbias, c, TPCp, gv)) {
                 if (wd.tick(kWDutySilu, i)) break;
-                if (backoff) __nanosleep(400);
+                __nanosleep(400);
               }
               while (!prog_prev8(pr, pbias, K + c, TPCp, uv)) {
                 if (wd.tick(kWDutySilu, i)) break;
-                if (backoff) __nanosleep(400);
+                __nanosleep(400);
               }
             } else {
               gv = ldcg_u4(o->src + c);
@@ -465,9 +462,8 @@ __global__ void __launch_bounds__(kProgThreads, 1)
     const int K = o->K, N = o->N, G = o->G, g_shift = o->g_shift;
     const int TPC = K / kV3TileRows;
     const int T = (N / kV3TileCols) * TPC;
-    const int np = o->n_part > 0 ? o->n_part : nblk;
-    const int t0 = bid < np ? (int)((int64_t)T * bid / np) : 0;
-    const int t1 = bid < np ? (int)((int64_t)T * (bid + 1) / np) : 0;
+    const int t0 = (int)((int64_t)T * bid / nblk);
+    const int t1 = (int)((int64_t)T * (bid + 1) / nblk);
     const int ntile = t1 - t0;
     const int a_w = t0 + (int)((int64_t)ntile * cw / kV3Warps);
     const int b_w = t0 + (int)((int64_t)ntile * (cw + 1) / kV3Warps);
@@ -768,7 +764,8 @@ static bool stream_build(Program* pr, const std::vector<ProgOp>& table, int grid
     max_cols = std::max(max_cols, (size_t)(mode[i] ? p.N / 2 : p.N));
     max_K = std::max(max_K, p.K);
   }
-  if (sp_fixed_smem(12, 3) + (size_t)max_K * 2 > (size_t)227 * 1024) return false;   // (the largest configuration)
+  // K <= 24160: the envelope is sized for 12 consumer warps x 3 stages, more than the 8-warp kernel needs
+  if (sp_fixed_smem(12, 3) + (size_t)max_K * 2 > (size_t)227 * 1024) return false;
   for (int i = 0; i < n; ++i) {
     const ProgOp& p = table[i];
     SpOp& o = ops[i];
@@ -838,10 +835,6 @@ static bool stream_build(Program* pr, const std::vector<ProgOp>& table, int grid
   if (e == cudaSuccess) e = cudaMemcpy(pr->d_cta, cta.data(), cta.size() * sizeof(uint32_t), cudaMemcpyHostToDevice);
   if (e == cudaSuccess)
     e = cudaFuncSetAttribute(stream_program_kernel<8, 4, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(227 * 1024));
-  if (e == cudaSuccess)
-    e = cudaFuncSetAttribute(stream_program_kernel<12, 3, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(227 * 1024));
-  if (e == cudaSuccess)
-    e = cudaFuncSetAttribute(stream_program_kernel<16, 2, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(227 * 1024));
   if (e == cudaSuccess) e = cudaDeviceSynchronize();
   if (e != cudaSuccess) {
     cudaFree(pr->d_stream);
@@ -961,12 +954,6 @@ int program_create(const b200awq_op_t* ops, int n, Program** out, cudaError_t* c
     p.K = op.K;
     p.N = op.N;
     p.G = op.group_size;
-    if (knob(13) > 0) {
-      const int tiles = (op.N / kV3TileCols) * (op.K / kV3TileRows);
-      int np = tiles / knob(13);
-      if (np < 1) np = 1;
-      p.n_part = np < grid ? np : 0;
-    }
     p.g_shift = 31;
     if ((p.G & (p.G - 1)) == 0) {
       p.g_shift = 0;
@@ -1055,8 +1042,6 @@ int program_create(const b200awq_op_t* ops, int n, Program** out, cudaError_t* c
   if (e == cudaSuccess) e = cudaMalloc(&pr->d_done, 2 * (table.size() + 1) * sizeof(int));
   if (e == cudaSuccess) e = cudaMemcpy(pr->d_ops, table.data(), table.size() * sizeof(ProgOp), cudaMemcpyHostToDevice);
   if (e == cudaSuccess)
-    e = cudaFuncSetAttribute(program_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(227 * 1024));
-  if (e == cudaSuccess)
     e = cudaFuncSetAttribute(program_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(227 * 1024));
   if (e != cudaSuccess) {
     cudaFree(pr->d_ops);
@@ -1081,14 +1066,12 @@ cudaError_t program_run(Program* p, float* acc_ws, cudaStream_t st) {
   cudaError_t e = program_abort_clear(st);
   if (e != cudaSuccess) return e;
   if (p->stream) {
-    // knob 9: consumer warps of the stream kernel: 8 (4 ring stages each, 4 units in flight; the default: measured
-    // best, 1.50 / 1.59 / 1.73 ms per Llama-3-8B step with 8 / 12 / 16), 12 (3 stages, 2 units) or 16 (2 stages, 2 units)
-    const int nw = knob(9) == 12 ? 12 : (knob(9) == 16 ? 16 : 8);
-    const int spw = nw == 8 ? 4 : (nw == 12 ? 3 : 2);
+    // 8 consumer warps, 4 ring stages each, 4 units in flight (measured 1.50 / 1.59 / 1.73 ms per Llama-3-8B step with
+    // 8 / 12 / 16 warps)
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(prog_sm_count());
-    cfg.blockDim = dim3(32 + nw * 32);
-    cfg.dynamicSmemBytes = sp_fixed_smem(nw, spw) + p->xs_bytes;
+    cfg.blockDim = dim3(32 + 8 * 32);
+    cfg.dynamicSmemBytes = sp_fixed_smem(8, 4) + p->xs_bytes;
     cfg.stream = st;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeCooperative;   // all CTAs co-resident: the hand-off polls are grid-wide waits
@@ -1097,28 +1080,15 @@ cudaError_t program_run(Program* p, float* acc_ws, cudaStream_t st) {
     cfg.numAttrs = 1;
     const SpOp* sops = p->d_sp_ops;
     const uint32_t* cta = p->d_cta;
-    // knob 8: HBM -> L2 prefetch window per producer lane in KB (<= 0 = off, the default: it helps only when the weight
-    // stream is the bottleneck - 1041 -> 895 us without the unit math - and costs 1-6 % with it)
-    const int l2_ahead = knob(8) <= 0 ? 0 : knob(8) * 1024;
-    // knob 10: ops ahead of the consumers' staging for which shared-memory loads may already be issued (0 = ungated,
-    // the default; n > 0: at most n - 1 ops ahead, 1 = strictly gated)
-    const int gate_ahead = knob(10) <= 0 ? 1 << 20 : knob(10) - 1;
-    if (nw == 8)
-      return cudaLaunchKernelEx(&cfg, stream_program_kernel<8, 4, 4>, sops, cta, p->n_ops, p->d_rows, p->row_stride,
-                                p->d_state, knob(3), l2_ahead, gate_ahead);
-    if (nw == 16)
-      return cudaLaunchKernelEx(&cfg, stream_program_kernel<16, 2, 2>, sops, cta, p->n_ops, p->d_rows, p->row_stride,
-                                p->d_state, knob(3), l2_ahead, gate_ahead);
-    return cudaLaunchKernelEx(&cfg, stream_program_kernel<12, 3, 2>, sops, cta, p->n_ops, p->d_rows, p->row_stride,
-                              p->d_state, knob(3), l2_ahead, gate_ahead);
+    return cudaLaunchKernelEx(&cfg, stream_program_kernel<8, 4, 4>, sops, cta, p->n_ops, p->d_rows, p->row_stride,
+                              p->d_state, knob(3));
   }
   e = cudaMemsetAsync(p->d_done, 0, (size_t)2 * (p->n_ops + 1) * sizeof(int), st);
   if (e != cudaSuccess) return e;
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(prog_sm_count());
   cfg.blockDim = dim3(kProgThreads);
-  const int spw = knob(9) == 1 ? 1 : 2;
-  cfg.dynamicSmemBytes = prog_fixed_smem(spw) + p->xs_bytes;
+  cfg.dynamicSmemBytes = prog_fixed_smem(2) + p->xs_bytes;
   cfg.stream = st;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeCooperative;   // all CTAs co-resident: the completion counters are grid-wide waits
@@ -1126,16 +1096,11 @@ cudaError_t program_run(Program* p, float* acc_ws, cudaStream_t st) {
   cfg.attrs = attr;
   cfg.numAttrs = 1;
   const ProgOp* ops = p->d_ops;
-  const int dbg = knob(3), gate = knob(10) == 2 ? 0 : 1;   // gate on unless knob 10 == 2
+  const int dbg = knob(3);
   unsigned long long* rows = reinterpret_cast<unsigned long long*>(acc_ws);
   int* staged = p->d_done;
   int* zeroed = p->d_done + (p->n_ops + 1);
-  const int backoff = knob(11) == 2 ? 0 : 1;   // duty-warp polls sleep 400 ns between attempts unless knob 11 == 2
-  if (spw == 1)
-    return cudaLaunchKernelEx(&cfg, program_kernel<1>, ops, p->n_ops, rows, p->acc_stride, staged, zeroed, p->M, dbg, gate,
-                              backoff);
-  return cudaLaunchKernelEx(&cfg, program_kernel<2>, ops, p->n_ops, rows, p->acc_stride, staged, zeroed, p->M, dbg, gate,
-                            backoff);
+  return cudaLaunchKernelEx(&cfg, program_kernel<2>, ops, p->n_ops, rows, p->acc_stride, staged, zeroed, p->M, dbg);
 }
 
 void program_destroy(Program* p) {

@@ -25,7 +25,6 @@
 
 namespace b200awq {
 
-constexpr int kSpMaxWarps = 16;                   // consumer warps at most (the kernel is a template over the count)
 constexpr int kSpStageWarps = 8;                  // warps that stage the activations (thread -> k mapping of aux.cu's
                                                   // rmsnorm_kernel: 256 threads x 8 consecutive k per pass)
 constexpr int kSpStagePass = kSpStageWarps * 32 * 8;   // k covered by one staging pass
@@ -58,8 +57,7 @@ __host__ __device__ constexpr size_t sp_fixed_smem(int nw, int spw) {
   return (size_t)nw * spw * kSpStageBytes + (size_t)kSpLMax * nw * 16 * 4 + (size_t)kSpXsumMax * 4 +
          (size_t)2 * nw * spw * 8 + 2 * 128 + 256;
 }
-static_assert(sp_fixed_smem(8, 4) % 16 == 0 && sp_fixed_smem(12, 3) % 16 == 0 && sp_fixed_smem(16, 2) % 16 == 0,
-              "xs must stay 16-byte aligned");
+static_assert(sp_fixed_smem(8, 4) % 16 == 0, "xs must stay 16-byte aligned");
 
 __device__ __forceinline__ uint4 ld_relaxed_u4(const void* p) {
   uint4 r;
@@ -68,14 +66,6 @@ __device__ __forceinline__ uint4 ld_relaxed_u4(const void* p) {
 }
 __device__ __forceinline__ void st_relaxed_u32(void* p, uint32_t v) {
   asm volatile("st.relaxed.gpu.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-}
-__device__ __forceinline__ void st_release_cta_smem(int* p, int v) {
-  asm volatile("st.release.cta.shared.s32 [%0], %1;" ::"r"(smem_u32(p)), "r"(v) : "memory");
-}
-__device__ __forceinline__ int ld_acquire_cta_smem(const int* p) {
-  int v;
-  asm volatile("ld.acquire.cta.shared.s32 %0, [%1];" : "=r"(v) : "r"(smem_u32(p)) : "memory");
-  return v;
 }
 __device__ __forceinline__ uint32_t sp_tag(int base, int op) { return (uint32_t)((base + op) % 65535 + 1); }
 
@@ -284,8 +274,7 @@ __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wai
 template <int NW, int SPW, int GR>
 __global__ void __launch_bounds__(32 + NW * 32, 1)
     stream_program_kernel(const SpOp* __restrict__ ops, const uint32_t* __restrict__ cta_all, int n_ops,
-                          uint32_t* __restrict__ rows, int row_stride, int* __restrict__ state, int dbg, int l2_ahead,
-                          int gate_ahead) {
+                          uint32_t* __restrict__ rows, int row_stride, int* __restrict__ state, int dbg) {
   extern __shared__ __align__(1024) uint8_t sp_smem[];
   uint8_t* ring = sp_smem;
   float* part = reinterpret_cast<float*>(sp_smem + (size_t)(NW * SPW) * kSpStageBytes);   // [LMax][8 warps][16]
@@ -298,8 +287,7 @@ __global__ void __launch_bounds__(32 + NW * 32, 1)
   int* wfirst = misc + 8;                              // [NW] first local set each warp touched (-1: none)
   int* wlast = misc + 8 + NW;                    // [NW]
   uint32_t* scta = reinterpret_cast<uint32_t*>(misc + 8 + 2 * NW);   // [2][2] this CTA's unit range (with sdesc)
-  int* staged_op = misc + 12 + 2 * NW;                 // last op this CTA staged (release / acquire at CTA scope)
-  static_assert((13 + 2 * NW) * 4 <= 256, "misc area");
+  static_assert((12 + 2 * NW) * 4 <= 256, "misc area");
   uint32_t* xs = reinterpret_cast<uint32_t*>(sp_smem + sp_fixed_smem(NW, SPW));   // activations in B-fragment order
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -312,7 +300,6 @@ __global__ void __launch_bounds__(32 + NW * 32, 1)
       mbar_init(&empty[s], 1);
     }
     fence_mbar_init();
-    *staged_op = -1;
   }
   if (warp == 1) {   // op 0's descriptor
     reinterpret_cast<uint32_t*>(sdesc)[lane] = reinterpret_cast<const uint32_t*>(ops)[lane];
@@ -353,15 +340,8 @@ __global__ void __launch_bounds__(32 + NW * 32, 1)
       int op = 0;
       fetch(0, cur);
       fetch(1, nxt);
-      // HBM -> L2 prefetch cursor, running ahead of the ring by at most `l2_ahead` bytes per lane: while the
-      // consumers hand activations from op to op the ring is full and HBM would idle; with the next chunks already in
-      // L2 the ring refills at L2 speed afterwards (the weights of ~1.5 ops fit: 148 x 8 lanes x l2_ahead)
-      Run pcur, pnxt;
-      int pop = 0;
-      fetch(0, pcur);
-      fetch(1, pnxt);
-      bool pactive = lane < NW && l2_ahead > 0;
-      int ahead = 0;                               // bytes prefetched beyond the ring's load cursor
+      // Loads are neither gated on the consumers' staging nor preceded by an HBM -> L2 prefetch: both measured slower
+      // here (DESIGN.md §3.5b, profiles/r02_stream_experiments.md).
       int stage_i = 0;
       uint32_t ph = 0;
       ProgWatch wd;
@@ -376,11 +356,7 @@ __global__ void __launch_bounds__(32 + NW * 32, 1)
         }
         if (!__any_sync(0xffffffffu, active)) break;
         bool issued = false;
-        // Gate: shared-memory loads of an op start only once this CTA has staged that op's activations (+ gate_ahead
-        // ops).  A deep ring of bulk loads is also a deep queue on the SM's return path: every poll of the hand-off
-        // waited behind ~100 KB of weight tiles (measured: 1.3 us per L2 round trip against 0.13 us unloaded).  While
-        // the consumers hand over, the stream continues into L2 (prefetch cursor below), not into this SM.
-        if (active && (gate_ahead >= (1 << 20) || op <= ld_acquire_cta_smem(staged_op) + gate_ahead)) {
+        if (active) {
           const int stage = w * SPW + stage_i;
           if (mbar_test_wait(&empty[stage], ph ^ 1)) {
             const int n = (int)(cur.ub - cur.u) < cur.ups ? (int)(cur.ub - cur.u) : cur.ups;
@@ -388,42 +364,13 @@ __global__ void __launch_bounds__(32 + NW * 32, 1)
             bulk_load_1d(ring + (size_t)stage * kSpStageBytes, cur.src + (size_t)cur.u * cur.UB, (uint32_t)(n * cur.UB),
                          &full[stage]);
             cur.u += (uint32_t)cur.ups;
-            ahead -= n * cur.UB;
             if (++stage_i == SPW) { stage_i = 0; ph ^= 1; }
             issued = true;
           }
         }
-        if (!__any_sync(0xffffffffu, issued)) {
-          // nothing to load: prefetch one more chunk into L2 if the window allows, else leave the issue slots alone
-          bool pf = false;
-          if (pactive) {
-            if (ahead < 0) {                       // the ring overtook the prefetch cursor: catch up
-              pop = op;
-              pcur = cur;
-              pnxt = nxt;
-              ahead = 0;
-            }
-            while (pactive && pcur.u >= pcur.ub) {
-              if (++pop >= n_ops) {
-                pactive = false;
-                break;
-              }
-              pcur = pnxt;
-              fetch(pop + 1, pnxt);
-            }
-            if (pactive && ahead < l2_ahead) {
-              const int n = (int)(pcur.ub - pcur.u) < pcur.ups ? (int)(pcur.ub - pcur.u) : pcur.ups;
-              // (chunks still inside the ring window were loaded already: prefetching them again is harmless)
-              bulk_prefetch_l2(pcur.src + (size_t)pcur.u * pcur.UB, (uint32_t)(n * pcur.UB));
-              pcur.u += (uint32_t)pcur.ups;
-              ahead += n * pcur.UB;
-              pf = true;
-            }
-          }
-          if (!__any_sync(0xffffffffu, pf)) {
-            if (__any_sync(0xffffffffu, wd.tick(kWEmpty, op))) break;   // watchdog (warp-uniform): never hang the GPU
-            __nanosleep(32);
-          }
+        if (!__any_sync(0xffffffffu, issued)) {   // nothing to load: leave the issue slots alone
+          if (__any_sync(0xffffffffu, wd.tick(kWEmpty, op))) break;   // watchdog (warp-uniform): never hang the GPU
+          __nanosleep(32);
         }
       }
     }
@@ -517,7 +464,6 @@ __global__ void __launch_bounds__(32 + NW * 32, 1)
                   if ((a.x >> 16) == want && (a.y >> 16) == want && (a.z >> 16) == want && (a.w >> 16) == want &&
                       (d.x >> 16) == want && (d.y >> 16) == want && (d.z >> 16) == want && (d.w >> 16) == want)
                     break;
-                  if (dbg == 6 || dbg == 7) break; // experiment: do not wait for the producers (results are garbage)
                   if (wd.tick(kWCopy, op)) break;
                   v0[b] = ld_relaxed_u4(row + c);
                   v1[b] = ld_relaxed_u4(row + c + 4);
@@ -585,7 +531,6 @@ __global__ void __launch_bounds__(32 + NW * 32, 1)
         }
         named_bar_sync_gv(1, (NW * 32));
       }
-      if (ct == 0) st_release_cta_smem(staged_op, op);      // releases the producer's loads of this op (see the gate)
       SP_STAMP(2);
       SP_TOUCH_SMEM();
       SP_WSTAMP(2);
@@ -623,21 +568,19 @@ __global__ void __launch_bounds__(32 + NW * 32, 1)
             SP_WSTAMP(3);
           }
           const uint8_t* st = ring + (size_t)stage * kSpStageBytes;
-          if (dbg != 5 && dbg != 7) {      // (5 / 7: experiment without the unit math)
-            auto apply = [&](float t_lo, float t_hi) {
-              ylo += t_lo;
-              yhi += t_hi;
-              if (++j == NU) {
-                flush();
-                j = 0;
-                ++s_cur;
-              }
-            };
-            const int j0 = j;
-            if (F == 8) sp_chunk<8, GR>(st, UB, n, xs, xsum, j0, NU, lane, xl, apply);
-            else if (F == 4) sp_chunk<4, GR>(st, UB, n, xs, xsum, j0, NU, lane, xl, apply);
-            else sp_chunk<2, GR>(st, UB, n, xs, xsum, j0, NU, lane, xl, apply);
-          }
+          auto apply = [&](float t_lo, float t_hi) {
+            ylo += t_lo;
+            yhi += t_hi;
+            if (++j == NU) {
+              flush();
+              j = 0;
+              ++s_cur;
+            }
+          };
+          const int j0 = j;
+          if (F == 8) sp_chunk<8, GR>(st, UB, n, xs, xsum, j0, NU, lane, xl, apply);
+          else if (F == 4) sp_chunk<4, GR>(st, UB, n, xs, xsum, j0, NU, lane, xl, apply);
+          else sp_chunk<2, GR>(st, UB, n, xs, xsum, j0, NU, lane, xl, apply);
           __syncwarp();
           if (lane == 0) mbar_arrive(&empty[stage]);
           if (++stage_i == SPW) { stage_i = 0; ph ^= 1; }

@@ -125,7 +125,8 @@ int b200awq_grouped_gemm_forward(const void* x, int x_rows_per_token, const int3
  * (M <= 128, G >= 64, K % 128 == 0, N % 128 == 0). */
 int b200awq_tcq_plan(int M, int K, int N, int group_size, int sm_count, int mode, int* grid, int* pairs_per_tile);
 
-/* Tuning / debug knobs (process-global; used by the micro-benchmarks and layout self-tests).
+/* Tuning / debug knobs (process-global; used by the micro-benchmarks and layout self-tests).  Keys not listed here
+ * are rejected with B200AWQ_EINVAL.
  *   key 0: GEMV rows per warp override: 32 / 64 / 128 (0 = heuristic)
  *   key 1: tensor-core path split-K override (0 = heuristic)
  *   key 2: M threshold at or below which the GEMV kernels are used (default 8; the GEMM-layout entry point lowers it to 4
@@ -147,31 +148,14 @@ int b200awq_tcq_plan(int M, int K, int N, int group_size, int sm_count, int mode
  *   key 6: 1 = enable the learned next-weight L2 prefetch (the M <= 8 path remembers which weight tensor
  *          followed which in the call sequence and prefetches the successor's packed weights into L2 at the
  *          tail of each kernel); default 0 - it measured slightly slower on B200
- *   key 7: 1 = stage the activations in shared memory in the persistent GEMV (M <= 2); default 0
- *   key 8: persistent GEMV L2-prefetch distance + 1 in tiles (0 / 1 = off, the default)
- *   key 9: persistent GEMV ring stages per consumer warp for M = 1 (1 / 2; 0 = default 3); the decode-program
- *          kernel uses 1 stage per warp when this is 1 (default 2)
- *   key 10: decode program: 2 = do NOT hold the next op's weight loads back until the CTA has pushed its sums of
- *           the previous op (default: hold them back, +9 % measured)
- *   key 11: decode program: 2 = no back-off in the duty warp's polls (default: 400 ns sleep between attempts)
  *   key 12: 2 = grouped_gemm_forward always uses the register-staged grouped kernel
- *   key 13: decode program (read at b200awq_program_create): minimum tiles per participating CTA; ops with fewer
- *           tiles per CTA are shared by fewer CTAs (0 = every CTA takes part in every op, the default: measured best)
- *   key 18: 1 = the persistent GEMV uses round 1's split-K epilogue (fp32 REDs, tickets, read-back) also at M = 1,
- *           instead of the packed one (one returning 64-bit atomic per element; bit-reproducible)
- *   key 17: 1 = b200awq_comm_all_reduce uses the flag protocol (push, fence, flag, wait, reduce) instead of the default
- *           LL protocol (8-byte words carrying {2 x fp16, call number}: one NVLink hop, no fences)
  *   key 16: decode-program watchdog in seconds (0 = the default 0.5 s): every spin of the program kernels gives up
  *           after this long; raise it under compute-sanitizer / a debugger, where kernels run orders of magnitude slower
  *   key 15: 1 = wrap every launching entry point in an NVTX range named after it (profiler timelines); default 0
  *   key 19: 1 = never use the small-M kernel with TMA-staged packed weights (gemm_tcq_kernel; default: every GEMM-layout
  *           call with 5 <= M <= 128 (M above key 2's threshold), G >= 64, K % 128 == 0, N % 128 == 0 runs it)
- *   key 20: small-M kernel timing experiments (outputs are WRONG while set): bit 0 = producers skip the dequantisation and
- *           the shared-memory stores, bit 1 = producers skip the generic->async proxy fence, bit 2 = no MMA is
- *           issued (commits only), bit 3 = one MMA per k-step instead of four
  *   key 21: small-M kernel work cut: 0 = tile-aligned ranges when N / 128 <= SM count (or from 64 tokens on), balanced
  *           (n-tile, k-step pair) ranges otherwise; 1 = always balanced; 2 = tile-aligned whenever possible
- *   key 22: small-M kernel: HBM -> L2 prefetch distance in k-step pairs ahead of the shared-memory ring (0 = off, default)
  *   key 14: decode program kind (read at b200awq_program_create): 0 = stream variant when the sequence fits it,
  *           else the split-K kernel; 1 = split-K kernel only; 2 = stream variant only
  */
@@ -234,8 +218,8 @@ int b200awq_program_destroy(b200awq_program_t prog);
  * One-shot all-reduce over NVLink peer memory (csrc/comm.cu; SURVEY 8e: the reference has no collective at all -
  * multi-GPU there is accelerate layer placement, awq/models/base.py:527-535).  For the tensor-parallel decode path:
  * the fp16 partial outputs of a row-parallel linear (o_proj / down_proj split along K) are summed across the GPUs
- * of one box in ONE kernel launch per call: push into every rank's inbox (P2P stores), flag, wait, reduce in rank
- * order (bit-identical results on all ranks).  One process per GPU: create -> exchange the 64-byte IPC handles by
+ * of one box in ONE kernel launch per call: push into every rank's inbox as words tagged with the call number (P2P
+ * stores), wait for the peers' words, reduce in rank order (bit-identical results on all ranks).  One process per GPU: create -> exchange the 64-byte IPC handles by
  * any means (autoawq_b200/comm.py uses torch.distributed.all_gather_object) -> open -> all_reduce any number of
  * times (asynchronous on `stream`, CUDA-graph capturable: the call counter lives on the device).  n % 8 == 0,
  * n <= max_elems (larger messages: use NCCL), world <= 8, y 16-byte aligned; in place.  b200awq_comm_error

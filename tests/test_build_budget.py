@@ -13,7 +13,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 @pytest.mark.skipif(shutil.which("nvcc") is None, reason="needs nvcc")
-def test_program_kernel_register_and_spill_budget(tmp_path):
+def test_program_kernels_register_and_spill_budget(tmp_path):
     src = os.path.join(ROOT, "autoawq_b200", "csrc", "program.cu")
     out = subprocess.run(
         ["nvcc", "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo", "-Xptxas", "-v", "-c", src,
@@ -22,8 +22,8 @@ def test_program_kernel_register_and_spill_budget(tmp_path):
     log = out.stderr + out.stdout
     entries = re.findall(r"Compiling entry function '(\S*program_kernel\S*)'[^\n]*\n[^\n]*\n\s*(\d+) bytes stack frame, "
                          r"(\d+) bytes spill stores, (\d+) bytes spill loads\n[^\n]*Used (\d+) registers", log)
-    assert len(entries) == 5, log[-1500:]          # program_kernel<1>, <2>, stream_program_kernel<8|12|16 warps>
-    assert sum("stream_program_kernel" in e[0] for e in entries) == 3
+    assert len(entries) == 2, log[-1500:]          # program_kernel<2>, stream_program_kernel<8 warps>
+    assert sum("stream_program_kernel" in e[0] for e in entries) == 1
     for name, stack, st, ld, regs in entries:
         if "stream_program_kernel" in name:
             # one resident CTA of 32 + 32 NW threads; a few spilled words in the staging phase (off the unit loop) are

@@ -134,6 +134,10 @@ def test_cabi_argument_validation_without_gpu(built):
     assert lib.b200awq_gemm_forward(None, 4096, None, None, None, None, None, 0, 4096, 4096, 128, None, 0, None) == 0
     assert lib.b200awq_dequantize_gemm(None, None, None, None, 128, 64, 128, None) == 1
     assert lib.b200awq_set_knob(99, 1) == 1 and lib.b200awq_get_knob(2) == 8
+    for retired in (7, 8, 9, 10, 11, 13, 17, 18, 20, 22):   # variants removed: a stale setting must fail loudly
+        assert lib.b200awq_set_knob(retired, 1) == 1 and lib.b200awq_get_knob(retired) == 0, retired
+    assert lib.b200awq_set_knob(12, 2) == 0 and lib.b200awq_get_knob(12) == 2
+    assert lib.b200awq_set_knob(12, 0) == 0
 
 
 # ------------------------------------------------------------------------------- C oracle

@@ -163,39 +163,10 @@ def bench_gemv_knobs():
     return res
 
 
-def bench_ring_sweep():
-    """Persistent GEMV, M = 1: ring depth (knob 9) x L2 prefetch distance (knob 8) on the four Llama shapes."""
-    res = {}
-    G = 128
-    for (K, N) in [(4096, 4096), (4096, 6144), (4096, 28672), (14336, 4096)]:
-        wbytes = K * N // 2 + (K // G) * N * 2 + (K // G) * N // 2
-        nbuf = max(3, int(400e6 // wbytes) + 1)
-        qw = [torch.randint(-2**31, 2**31 - 1, (K, N // 8), dtype=torch.int32, device=dev) for _ in range(nbuf)]
-        qz = [torch.randint(-2**31, 2**31 - 1, (K // G, N // 8), dtype=torch.int32, device=dev) for _ in range(nbuf)]
-        sc = [(torch.rand((K // G, N), device=dev) * 0.01 + 0.001).half() for _ in range(nbuf)]
-        x = torch.randn((1, K), device=dev, dtype=torch.float16)
-        ext.set_knob(4, 1)
-        for spw in (1, 2, 3):
-            for pf in (1, 3, 7):  # knob value = distance + 1
-                ext.set_knob(9, spw if spw < 3 else 0)
-                ext.set_knob(8, pf)
-                us = time_kernel(lambda i: ext.linear_forward("gemm", x, qw[i], sc[i], qz[i], G), nbuf, iters=200, warm=10)
-                res[f"K{K}_N{N}_spw{spw}_l2ahead{pf - 1}"] = round(us, 2)
-        ext.set_knob(9, 0)
-        ext.set_knob(8, 0)
-        ext.set_knob(4, 0)
-        del qw, qz, sc
-        torch.cuda.empty_cache()
-    return res
-
-
 if __name__ == "__main__":
     os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
     out["checks"] = check_paths()
     print(json.dumps(out["checks"], indent=1), flush=True)
-    if "--ring" in sys.argv:
-        out["ring_sweep"] = bench_ring_sweep()
-        print(json.dumps(out["ring_sweep"], indent=1), flush=True)
     if "--knobs" in sys.argv:
         out["gemv_knobs"] = bench_gemv_knobs()
         print(json.dumps(out["gemv_knobs"], indent=1), flush=True)

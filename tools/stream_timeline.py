@@ -15,7 +15,7 @@ from autoawq_b200._cabi import lib  # noqa: E402
 from autoawq_b200.program import DecodeProgram  # noqa: E402
 
 dev = torch.device("cuda:0")
-for kv in sys.argv[1:]:      # KEY=VALUE library knobs, e.g. 8=-1 10=1 9=8
+for kv in sys.argv[1:]:      # KEY=VALUE library knobs, e.g. 14=2 (no fall-back to the split-K kernel)
     k, v = kv.split("=")
     ext.set_knob(int(k), int(v))
 print("knobs:", sys.argv[1:])
